@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — UAHN image-pair inferences/sec on N B200 (BASELINE.json metric) + p50 batch-1 latency.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--precision bf16|fp32] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (3-block UAHN with EKF prior: prior DLT, blocks 2,3 and the
 uncertainty block 4, covariance transfer) over the workload of BASELINE.json configs[3]: 8192 synthetic pairs,
@@ -17,6 +17,10 @@ C-ABI call (pinned host inputs, H2D + D2H inside the timed region) with the bare
 config3_256_pairs = BASELINE.json configs[2] (256 pairs in one infer_batch) with its own roofline;
 latency_batch1 = configs[1] in bf16 AND fp32; streaming_show_error = configs[4];
 cpu_baseline = the reference's own TorchScript graphs (oracle/_ref) on the host cores (all threads, 1 thread, twins).
+
+Every timed pass (value, the profiled pass, config3_256_pairs, e2e, its copy ceiling, e2e_independent_pairs) runs
+exactly K = --steps steps; the JSON reports K with each.  A run with a few steps rests on a few calls (config3_256_pairs
+on K calls of about 0.7 ms), so compare only runs with the same --steps; the default is 20.
 """
 from __future__ import annotations
 
@@ -59,7 +63,30 @@ def parse():
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline sample")
     ap.add_argument("--no-latency", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step (mean [pairs, 8], cov [pairs, 8, 8], float32, all ranks "
+                         "in rank order) as DIR/<name>.npy, to compare two builds output for output")
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
+
+
+DUMP_BYTES = 60 << 20      # one dump stays below 64 MB
+
+
+def dump_outputs(directory: str, arrays: dict):
+    """Write {name: array with one row per pair} as directory/<name>.npy.  Above DUMP_BYTES every array keeps the same
+    rows, a seeded sample in pair order, so two runs with the same arguments write the same pairs."""
+    import numpy as np
+    n = len(next(iter(arrays.values())))
+    per_pair = sum(a[:1].nbytes for a in arrays.values())
+    if n * per_pair > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // per_pair, replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -395,12 +422,13 @@ def run_ours(args):
     l0 = net.launch_count
     ms_max = timed_device(lambda i: step(W + i), K)
     launches = net.launch_count - l0
+    # the last timed step's results, before the passes below overwrite them
+    last = {"mean": mean.cpu().numpy(), "cov": cov.view(B, 8, 8).cpu().numpy()} if args.dump_outputs else None
     value = total_pairs * K / (ms_max * 1e-3)
     clk = clocks.stop() if clocks else None
     # ---- pass 2: per-stage CUDA events (uahn_profile_*) for the roofline and the stage split ----------------------
-    Kp = max(3, min(K, 10))
     net.profile_enable(True)
-    ms_prof = timed_device(lambda i: step(W + i), Kp)
+    ms_prof = timed_device(lambda i: step(W + i), K)
     prof_ms, prof_cnt = net.profile_read()
     net.profile_enable(False)
 
@@ -411,16 +439,15 @@ def run_ours(args):
         f0, p0 = sets[0]
         for i in range(W + 5):
             run_resident(f0, p0, n3, n3, base=(i % 8) * 16)
-        K3 = max(K, 20)
-        ms3 = timed_device(lambda i: run_resident(*sets[i % n_sets], n3, n3, base=(i % 8) * 16), K3)
+        ms3 = timed_device(lambda i: run_resident(*sets[i % n_sets], n3, n3, base=(i % 8) * 16), K)
         net.profile_enable(True)
-        timed_device(lambda i: run_resident(*sets[i % n_sets], n3, n3, base=(i % 8) * 16), K3)
+        timed_device(lambda i: run_resident(*sets[i % n_sets], n3, n3, base=(i % 8) * 16), K)
         p3, c3 = net.profile_read()
         net.profile_enable(False)
-        cfg3 = {"pairs_per_call": n3, "ms_per_call": ms3 / K3, "value": n3 * K3 / (ms3 * 1e-3), "unit": UNIT,
-                "stage_ms_per_call": {"warp_concat_pool": p3[0] / K3, "conv_stacks": p3[1] / K3, "mc_head_gemm": p3[2] / K3,
-                                      "fc_dlt_mc_small": p3[3] / K3},
-                "launches_per_call": int(sum(int(v) for v in c3) // K3)}
+        cfg3 = {"pairs_per_call": n3, "ms_per_call": ms3 / K, "value": n3 * K / (ms3 * 1e-3), "unit": UNIT,
+                "stage_ms_per_call": {"warp_concat_pool": p3[0] / K, "conv_stacks": p3[1] / K, "mc_head_gemm": p3[2] / K,
+                                      "fc_dlt_mc_small": p3[3] / K},
+                "launches_per_call": int(sum(int(v) for v in c3) // K)}
 
     # ---- e2e: host buffers through the C ABI, copies inside the timed region ---------------------------
     # The call a streaming user makes for a sequence: uahn_submit_sequence from pinned host memory — every frame crosses
@@ -449,8 +476,7 @@ def run_ours(args):
         torch.cuda.synchronize()
         return total_pairs * steps / (reduce_max_ms(1e3 * (time.perf_counter() - t0), dev) * 1e-3)
 
-    Ke = max(3, K)      # the same K steps; the last forward (not hidden behind a following copy) is part of the timed region
-    e2e_value = timed(step_e2e, Ke)
+    e2e_value = timed(step_e2e, K)      # the last forward (not hidden behind a following copy) is part of the timed region
     # results of the two paths must agree (same frames, priors, seed and pair indices)
     run_resident(torch.from_numpy(hf).to(dev), torch.from_numpy(hprior).to(dev))
     torch.cuda.synchronize()
@@ -476,9 +502,9 @@ def run_ours(args):
             copy_step(i)
         copy_stream.synchronize()
         return reduce_max_ms(1e3 * (time.perf_counter() - t0), dev) * 1e-3
-    t_copy = timed_copy(Ke)
-    h2d_gbs_all = world * (B + 1) * FR * Ke / t_copy / 1e9
-    ceiling_pairs = total_pairs * Ke / t_copy
+    t_copy = timed_copy(K)
+    h2d_gbs_all = world * (B + 1) * FR * K / t_copy / 1e9
+    ceiling_pairs = total_pairs * K / t_copy
     del dstage
 
     # ---- the same pairs submitted as INDEPENDENT pairs (uahn_submit_batch): prev and curr arrays are separate host
@@ -491,7 +517,15 @@ def run_ours(args):
             n = min(chunk, B - o)
             net.submit_batch_ptrs(n, php[o:].data_ptr(), phc[o:].data_ptr(), ppr[o:].data_ptr(), hmean[o:].data_ptr(),
                                   hcov[o:].data_ptr(), seed=1, first_pair=first0 + o)
-    e2e_pairs_value = timed(step_pairs, Ke)
+    e2e_pairs_value = timed(step_pairs, K)
+
+    if last is not None:
+        parts = [last]
+        if world > 1:
+            parts = [None] * world
+            dist.all_gather_object(parts, last)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {k: np.concatenate([p[k] for p in parts]) for k in last})
 
     if rank != 0:
         if world > 1:
@@ -520,12 +554,12 @@ def run_ours(args):
                 "launch_groups_per_step": calls,
                 "peak_source": f"MEASURED_PEAKS.json bf16_tflops_sustained ({peaks['source']})"}
 
-    conv_ms_per_call = prof_ms[1] / Kp / calls_per_step
-    warp_ms_per_step = prof_ms[0] / Kp
+    conv_ms_per_call = prof_ms[1] / K / calls_per_step
+    warp_ms_per_step = prof_ms[0] / K
     roof = tensor_roofline(conv_ms_per_call, chunk, calls_per_step)
     roof.update({"traffic": traffic, "traffic_source": traffic_src,
                  "hbm_frac_conv_group": (traffic / (conv_ms_per_call * 1e-3) / 1e9 / peaks["hbm_gbs"]) if traffic and conv_ms_per_call > 0 else None,
-                 "ms_per_step": prof_ms[1] / Kp, "timed_in": f"second pass of {Kp} steps with per-stage CUDA events on the launching stream"})
+                 "ms_per_step": prof_ms[1] / K, "timed_in": f"second pass of {K} steps with per-stage CUDA events on the launching stream"})
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
         "ms_per_step": ms_max / K, "higher_is_better": True, "scaling": args.scaling, "vs_baseline": None,
@@ -541,7 +575,7 @@ def run_ours(args):
                    "parallelism": f"independent pairs, {world} shard(s) from sharding.shard_range, no data-path collective",
                    "host_numa_binding_rank0": numa},
         "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": h2d_step,
-                "d2h_bytes_per_step": B * 72 * 4, "steps": Ke, "matches_device_path": same,
+                "d2h_bytes_per_step": B * 72 * 4, "steps": K, "matches_device_path": same,
                 "what": "uahn_submit_sequence + uahn_wait from pinned host buffers: the shard's consecutive frames, each "
                         "uploaded once per step (per-GPU byte counts)",
                 "h2d_ceiling": {"pairs_per_s": ceiling_pairs, "h2d_gbs_all_ranks": h2d_gbs_all,
@@ -550,17 +584,17 @@ def run_ours(args):
                 "h2d_ceiling_frac": e2e_value / ceiling_pairs if ceiling_pairs else None,
                 "bound": "device (resident rate)" if value <= ceiling_pairs else "host-to-device copy"},
         "e2e_independent_pairs": {"value": e2e_pairs_value, "unit": UNIT, "h2d_bytes_per_step": B * (2 * 71680 + 32),
-                                  "d2h_bytes_per_step": B * 72 * 4, "steps": Ke,
+                                  "d2h_bytes_per_step": B * 72 * 4, "steps": K,
                                   "what": "the same pairs through uahn_submit_batch with separate prev / curr host arrays "
                                           "(every frame crosses PCIe twice)"},
         "gpu_launches": int(launches),
         "clocks": clk,
         "roofline": roof,
-        "profiled_pass": {"steps": Kp, "ms_per_step": ms_prof / Kp, "note": "the pass the stage split and the roofline come from; "
+        "profiled_pass": {"steps": K, "ms_per_step": ms_prof / K, "note": "the pass the stage split and the roofline come from; "
                           "`value` is from the pass without profiling events"},
-        "stage_ms_per_step": {"warp_concat_pool": warp_ms_per_step, "conv_stacks": prof_ms[1] / Kp,
-                              "mc_head_gemm": prof_ms[2] / Kp, "fc_dlt_mc_small": prof_ms[3] / Kp},
-        "stage_launches_per_step": {k: int(v // Kp) for k, v in zip(("warp", "conv", "mc_gemm", "small"), prof_cnt)},
+        "stage_ms_per_step": {"warp_concat_pool": warp_ms_per_step, "conv_stacks": prof_ms[1] / K,
+                              "mc_head_gemm": prof_ms[2] / K, "fc_dlt_mc_small": prof_ms[3] / K},
+        "stage_launches_per_step": {k: int(v // K) for k, v in zip(("warp", "conv", "mc_gemm", "small"), prof_cnt)},
         "hbm": {"kernel": f"warp+concat+pool (3 texture-gather launches + the cell-array fill per call, {calls_per_step} call(s) per step; "
                           "the fill's time is inside, only the 3 warps are credited)",
                 "algorithmic_bytes_per_step": 3 * WARP_BYTES * B,

@@ -92,9 +92,9 @@ def dlt_solve(src: torch.Tensor, dst: torch.Tensor) -> torch.Tensor:
 
 
 def conv_lrelu(x, sd, key, stride):
-    """model_to_trace.py:7-15 — Conv2d(pad=(k-1)//2, bias) → LeakyReLU(0.1)."""
+    """model_to_trace.py:7-15 — Conv2d(pad=(k-1)//2, bias) → LeakyReLU(0.1, inplace)."""
     w = sd[key + ".0.weight"]
-    return F.leaky_relu(F.conv2d(x, w, sd[key + ".0.bias"], stride=stride, padding=(w.shape[-1] - 1) // 2), 0.1)
+    return F.leaky_relu(F.conv2d(x, w, sd[key + ".0.bias"], stride=stride, padding=(w.shape[-1] - 1) // 2), 0.1, True)
 
 
 BLOCK_LAYERS = {
@@ -182,7 +182,7 @@ def mc_head(f, sd, masks):
 
     def head(name, ma, mb):
         h = F.linear(x * ma, sd[P4 + name + ".1.weight"], sd[P4 + name + ".1.bias"])
-        h = F.leaky_relu(h, 0.1) * mb
+        h = F.leaky_relu(h, 0.1, True) * mb
         return F.linear(h, sd[P4 + name + ".4.weight"], sd[P4 + name + ".4.bias"]).view(MC, 4, 2)
 
     mean = head("fc_block_4_mean", m1, m2)
@@ -241,6 +241,44 @@ def forward(img1, img2, sd, masks, prior=None, show_error=False, blocks_to_run=3
             taps.mc_mean, taps.mc_logvar, taps.mu, taps.var, taps.H_total = mean, logvar, mu, var, Ht
             taps.H[4] = Hp
         return flow.reshape(8, 1), cov, err
+
+
+class TracedModel(torch.nn.Module):
+    """`combined_stu_model` (model_to_trace.py:284-330) as far as a TorchScript trace of it shows: the reference's
+    parameter tree (the 54 state_dict names, model_to_trace.py:333-350) around `forward` above, with fresh MC-dropout
+    masks on every call like the reference's train-mode nn.Dropout."""
+
+    def __init__(self, sd, show_error: bool = False, blocks_to_run: int = 3):
+        super().__init__()
+        for key, t in sd.items():
+            *path, leaf = key.split(".")
+            mod = self
+            for name in path:
+                if name not in mod._modules:
+                    mod.add_module(name, torch.nn.Module())
+                mod = mod._modules[name]
+            mod.register_parameter(leaf, torch.nn.Parameter(t.clone(), requires_grad=False))
+        self.show_error, self.blocks_to_run = show_error, blocks_to_run
+
+    def forward(self, img1, img2, prior=None):
+        masks = tuple(F.dropout(torch.ones(MC, n), 0.05, True) for n in (5120, 256, 5120, 256))
+        flow, cov, err = forward(img1, img2, dict(self.named_parameters()), masks, prior, self.show_error, self.blocks_to_run)
+        return (flow, cov) if err is None else (flow, cov, err)
+
+
+def trace(sd, variant: str = "prior3", show_error: bool = False):
+    """TorchScript of one reference graph, traced like trace_model.py:20-22,36-46 (check_trace=False), but of
+    `TracedModel`: the reference's `.pt` files without the reference's source.  tests/golden/reference_graphs.json
+    records, from the reference's own traces, the op-kind counts and inputs of the full and 3-block graphs (with and
+    without the error map) and the state_dict names; tests/test_weights.py holds these traces to that record.  The
+    2-block and 1-block graphs were not recorded."""
+    import contextlib
+    import io
+    blocks_to_run = {"full": 3, "prior3": 3, "prior2": 2, "prior1": 1}[variant]
+    img1, img2 = torch.ones(1, 1, IMG_H, IMG_W) * 0.2, torch.ones(1, 1, IMG_H, IMG_W) * 0.5
+    args = (img1, img2) if variant == "full" else (img1, img2, torch.ones(1, 1, 4, 2) * 0.9)
+    with torch.no_grad(), contextlib.redirect_stdout(io.StringIO()), contextlib.redirect_stderr(io.StringIO()):
+        return torch.jit.trace(TracedModel(sd, show_error, blocks_to_run), args, check_trace=False)
 
 
 def u8_to_unit(img_u8) -> torch.Tensor:
