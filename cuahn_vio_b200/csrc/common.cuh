@@ -54,7 +54,7 @@ struct ConvGeom {
 // previous kernel drains, and block in pdl_wait() until its memory is visible.  Nothing produced by an earlier
 // kernel may be read, and nothing may be written to global memory, before pdl_wait() — and EVERY kernel of the chain calls it,
 // even one that reads nothing from its predecessor: a grid that never waits could complete before the grid in front of it and
-// release its own dependents too early.  Used at every batch size (engine.cu: pdl_select); UAHN_NO_PDL=1 disables it.
+// release its own dependents too early.  Used at every batch size (engine.cu: pdl_enabled); UAHN_NO_PDL=1 disables it.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 // Grids that fit the machine in one wave (the latency path: 28-CTA warp bands, 32-CTA split-K clusters) let their dependents
@@ -101,7 +101,7 @@ struct SmemOptIn {   // one (function-local static) per kernel instantiation
   }
 };
 
-bool pdl_enabled();   // engine.cu: switched per forward() call by the batch size
+bool pdl_enabled();   // engine.cu: on for a thread once it has run a forward(), unless UAHN_NO_PDL is set
 template <typename... KArgs, typename... Args>
 cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg{};

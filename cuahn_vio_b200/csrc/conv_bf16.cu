@@ -630,21 +630,18 @@ int conv_bf16_prepare(ConvBf16Weights& wb, const std::vector<float>& wk, const s
                       const ConvGeom& g, const Tensor& in, const Tensor& out, std::vector<void*>& allocs,
                       std::string& err) {
   (void)out;
-  if (in.p) {   // block_2_1: the dedicated TMA-staged stride-2 first-layer kernel
+  if (in.p) {
+    // block_2_1: the dedicated TMA-staged stride-2 first-layer kernel; other convolutions: the shifted-window TMA kernels
     std::string serr;
-    const int rc = conv_s2first_prepare(wb.s2, wk, bias, g, in, allocs, serr);
+    int rc = conv_s2first_prepare(wb.s2, wk, bias, g, in, allocs, serr);
     if (rc < 0) { err = serr; return rc; }
-    // (the gather operands below are still built: they serve batches whose last tile the TMA path does not cover — none
-    //  today — and UAHN_NO_S2FIRST A/B runs)
-  }
-  if (in.p && !getenv("UAHN_NO_TMA")) {
-    std::string terr;
-    const int rc = conv_tma_prepare(wb.tma, wk, bias, g, in, allocs, terr);
-    if (rc < 0) { err = terr; return rc; }
+    if (wb.s2.enabled) { wb.ready = 1; return 0; }
+    rc = conv_tma_prepare(wb.tma, wk, bias, g, in, allocs, serr);
+    if (rc < 0) { err = serr; return rc; }
     if (wb.tma.enabled) { wb.ready = 1; return 0; }
   }
   // im2col TMA A producer: layers whose K stage is exactly one (tap, 64-channel chunk)
-  const bool im2col_ok = in.p && g.Cin % 64 == 0 && g.KH == g.KW && g.KH > 1 && !getenv("UAHN_NO_IM2COL");
+  const bool im2col_ok = in.p && g.Cin % 64 == 0 && g.KH == g.KW && g.KH > 1;
   const int xb = im2col_ok ? 1 : choose_xb(g);
   if (!xb) { err = "no valid Toeplitz factor"; return -1; }
   if (g.Cin % 8 && !(g.Cin == 2 && (xb * g.stride) % 4 == 0)) { err = "unsupported Cin"; return -1; }

@@ -370,10 +370,7 @@ int conv_tma_prepare(TmaPlan& plan, const std::vector<float>& wk, const std::vec
   plan.slot_bytes = (plan.slot_bytes + 1023) / 1024 * 1024;
   const int b_stages = g.KH * chunks;
   const size_t fixed = (n_total == 64 ? tma_smem_bytes<64>(0, 0, b_stages) : tma_smem_bytes<128>(0, 0, b_stages));
-  // UAHN_TMA_SMEM_RESERVE leaves shared memory free so CTAs of an ALU-bound kernel from another stream (the warp
-  // kernel of a second handle) can co-reside with this HBM-bound persistent kernel
-  const int reserve = getenv("UAHN_TMA_SMEM_RESERVE") ? atoi(getenv("UAHN_TMA_SMEM_RESERVE")) : 0;
-  int slots = (int)((SMEM_LIMIT - reserve - (int)fixed) / plan.slot_bytes);
+  int slots = (int)((SMEM_LIMIT - (int)fixed) / plan.slot_bytes);
   slots = std::min(slots, std::min(MAX_SLOTS, 3 * plan.n_planes));
   if (slots < plan.n_planes + 1 && slots < 2) return 0;
   plan.n_slots = slots;

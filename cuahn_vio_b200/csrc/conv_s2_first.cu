@@ -227,7 +227,6 @@ PFN_cuTensorMapEncodeTiled_v12000 get_encode_s2() {
 int conv_s2first_prepare(S2Plan& plan, const std::vector<float>& wk, const std::vector<float>& bias, const ConvGeom& g,
                          const Tensor& x, std::vector<void*>& allocs, std::string& err) {
   plan.enabled = 0;
-  if (getenv("UAHN_NO_S2FIRST")) return 0;
   if (!(g.KH == 7 && g.KW == 7 && g.stride == 2 && g.Cin == 2 && g.Cout == 64)) return 0;
   if (x.ph != 3 || x.pwl != 3 || x.C != 2 || g.Wo % 2) return 0;
   plan.Wog = g.Wo / 2;

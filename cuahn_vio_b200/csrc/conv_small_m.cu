@@ -13,7 +13,6 @@
 // with n & 7 — which is also conflict-free for ldmatrix), math is mma.sync.m16n8k16 bf16 with fp32 accumulation: 20-160 rows
 // cannot fill a 128-row UMMA tile, and the legacy path needs no TMEM allocation or descriptor set-up on a 4 us kernel.
 // The weight copies are issued BEFORE griddepcontrol.wait: they do not depend on the previous layer and overlap its tail.
-#include <cstdlib>
 
 #include "common.cuh"
 #include "conv_bf16.h"
@@ -200,8 +199,7 @@ cudaError_t launch_mt(const SmallMParams& p, cudaStream_t st) {
 
 // 1: this layer at this batch takes the split-K latency kernel
 int conv_small_m_ok(const ConvBf16Weights& wb, const ConvGeom& g) {
-  static const bool off = getenv("UAHN_NO_SMALL_M") != nullptr;
-  if (off || !wb.ready || wb.xb != 1 || g.Cin % 64 || g.Cout % SMM_NSLAB || g.KH != g.KW || wb.n_total != g.Cout) return 0;
+  if (!wb.ready || wb.xb != 1 || g.Cin % 64 || g.Cout % SMM_NSLAB || g.KH != g.KW || wb.n_total != g.Cout) return 0;
   const int k_stages = g.KH * g.KW * (g.Cin / 64);
   if (wb.k_total != k_stages * 64 || (k_stages + SMM_CLUSTER - 1) / SMM_CLUSTER > SMM_MAXCH) return 0;
   // worth it where the tcgen05 kernel would be a handful of CTAs walking a long K loop

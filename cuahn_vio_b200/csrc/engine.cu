@@ -19,20 +19,15 @@
 using namespace uahn;
 
 namespace uahn {
-// Programmatic dependent launch pays on the latency path (batch 1: 27 dependent kernels of a few microseconds each,
-// -9 % p50) and costs throughput on large batches (early-launched CTAs of the next kernel sit on the SMs of a
-// persistent kernel that still runs: -8 % at 1024 pairs), so forward() switches it per call.
+// Programmatic dependent launch at every batch size: with the next grid already resident in the launch queue its CTAs
+// start as SMs drain, which is worth 2-3 us per dependent kernel — 9 % of the batch-1 p50 (27 dependent kernels of a few
+// microseconds each), 10 % of a 256-pair call (0.748 -> 0.671 ms), 2 % of a 1024-pair call (same-box A/B on B200).
+// The flag is per thread and set by the first forward() on it: the stage entry points and the preprocessing launches of
+// a thread that has not run a forward yet go without.  UAHN_NO_PDL=1 disables it.
 static thread_local bool g_pdl_on = false;
 bool pdl_enabled() {
   static const bool allowed = getenv("UAHN_NO_PDL") == nullptr;
   return allowed && g_pdl_on;
-}
-// Every batch size (round 2; the first half of the round used it for <= 8 pairs only): with the next grid already resident in
-// the launch queue its CTAs start as SMs drain, which is worth 2-3 us per dependent kernel — 2 % of a 1024-pair call, 10 % of a
-// 256-pair call (0.748 -> 0.671 ms, same-box A/B).  UAHN_PDL_MAX_PAIRS=n restricts it to calls of at most n pairs.
-void pdl_select(int n_pairs) {
-  static const int max_pairs = getenv("UAHN_PDL_MAX_PAIRS") ? atoi(getenv("UAHN_PDL_MAX_PAIRS")) : (1 << 30);
-  g_pdl_on = n_pairs <= max_pairs;
 }
 }  // namespace uahn
 
@@ -114,7 +109,6 @@ struct Layer {
 struct Block {
   int id = 0, pool = 1;
   bool active = false;
-  int chunk_cap = 0;        // pairs held by x and layers[0].out (L2-resident chunking of the block front)
   FusedPlan fused;          // blocks 3/4 in bf16: conv 0 + conv 1 fused, conv 0's output never reaches HBM
   Tensor x_unfused;         // small halo-3 input used only by the per-layer stage entry point in fused mode
   Tensor x;                 // 2-channel conv input
@@ -179,10 +173,6 @@ struct uahn_handle {
   float* d_out1 = nullptr;      // device {mean[8], cov[64]} of uahn_infer
   uint64_t infer_calls = 0;
   bool use_graph = true;
-  // pairs per chunk of the block-3/4 fronts (UAHN_L2_CHUNK).  Measured on B200 at 1024 pairs/step: chunks of
-  // 16/32/64 pairs run the step 2.4x/1.65x/1.3x SLOWER than unchunked (launch + pipeline fill/drain of ~190 extra
-  // launches outweigh the saved HBM round trip), so chunking is off by default.
-  int l2_chunk = 1 << 30;
   // pipelined submissions (uahn_submit_batch): copy stream + second staging set
   cudaStream_t copy_stream = nullptr;
   cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
@@ -320,12 +310,8 @@ int build_block(uahn_handle* h, const std::map<std::string, HostTensor>& w, int 
   B.id = id; B.pool = pool; B.active = true;
   const char* pre = id == 4 ? P4 : P1;
   int H = IMG_H / pool, W = IMG_W / pool;
-  // Blocks 3 and 4: the warp output and the first conv's output are the largest activations (0.7 / 1.4 MB per
-  // pair).  They live in chunk-sized buffers that are re-used for every chunk of `l2_chunk` pairs, so the
-  // warp -> conv0 -> conv1 chain of a chunk runs out of L2 and those bytes never round-trip HBM.
-  B.chunk_cap = (id >= 3) ? std::min(h->cap, h->l2_chunk) : h->cap;
-  const bool try_fuse = h->bf16 && id >= 3 && B.chunk_cap == h->cap && !getenv("UAHN_NO_FUSE");
-  int rc = make_tensor(h, B.x, B.chunk_cap, H, W, 2, try_fuse ? 5 : (specs[0].k - 1) / 2);
+  const bool try_fuse = h->bf16 && id >= 3 && !getenv("UAHN_NO_FUSE");
+  int rc = make_tensor(h, B.x, h->cap, H, W, 2, try_fuse ? 5 : (specs[0].k - 1) / 2);
   if (rc) return rc;
   const int small_cap = std::min(h->cap, 4);
   if (try_fuse && (rc = make_tensor(h, B.x_unfused, small_cap, H, W, 2, (specs[0].k - 1) / 2))) return rc;
@@ -341,7 +327,7 @@ int build_block(uahn_handle* h, const std::map<std::string, HostTensor>& w, int 
     L.Wo = (W + 2 * p - L.spec.k) / L.spec.stride + 1;
     L.in = cur;
     const int next_pad = i + 1 < nl ? (specs[i + 1].k - 1) / 2 : 0;
-    rc = make_tensor(h, L.out, i == 0 ? (try_fuse ? small_cap : B.chunk_cap) : h->cap, L.Ho, L.Wo, L.spec.cout, next_pad);
+    rc = make_tensor(h, L.out, i == 0 && try_fuse ? small_cap : h->cap, L.Ho, L.Wo, L.spec.cout, next_pad);
     if (rc) return rc;
     const std::string key = std::string(pre) + L.spec.name + ".0.";
     const HostTensor* wt = find(w, key + "weight", {L.spec.cout, L.spec.cin, L.spec.k, L.spec.k}, err);
@@ -423,54 +409,38 @@ int build_head(uahn_handle* h, const std::map<std::string, HostTensor>& w) {
 }
 
 template <typename T>
-int run_conv(uahn_handle* h, Layer& L, int n, size_t out_img0 = 0) {
+int run_conv(uahn_handle* h, Layer& L, int n) {
   ConvGeom g = make_geom(L, n);
-  T* out = (T*)L.out.p + out_img0 * (size_t)L.out.pitch_n;     // first output image (chunked block fronts)
   if constexpr (sizeof(T) == 4) {
-    LAUNCH(launch_conv_f32((const float*)L.in.p, L.w_f32, L.bias, (float*)out, g, h->stream, n <= F32_SPLITK_MAX_PAIRS ? h->f32_ws : nullptr,
+    LAUNCH(launch_conv_f32((const float*)L.in.p, L.w_f32, L.bias, (float*)L.out.p, g, h->stream, n <= F32_SPLITK_MAX_PAIRS ? h->f32_ws : nullptr,
                            h->f32_ws_floats, L.Ho * L.Wo));
     h->launches += conv_f32_extra_launches();
   } else {
-    LAUNCH(launch_conv_bf16(L.wb, L.in.p, L.bias, out, g, h->stream));
+    LAUNCH(launch_conv_bf16(L.wb, L.in.p, L.bias, L.out.p, g, h->stream));
   }
   return UAHN_OK;
 }
 
-// warp + concat + pool -> conv stack of one cascade block.  The front (warp, conv 0, conv 1) runs per L2-sized chunk.
+// warp + concat + pool -> conv stack of one cascade block: the warp, then either the fused front (convs 0 and 1) and
+// layers 2.. or every layer in order.
 template <typename T>
 int run_block(uahn_handle* h, Block& B, int n, const uint8_t* prev, const uint8_t* curr, const float* Hcur,
               const WarpCells* cells = nullptr) {
   cudaStream_t st = h->stream;
   int rc;
-  const int CH = B.chunk_cap;
   const size_t nl = B.layers.size();
-  if (B.fused.enabled) {
-    if constexpr (sizeof(T) == 2) {
-      const int num_sms = h->num_sms;
-      h->prof_begin(0);
-      LAUNCH(launch_warp_concat_pool<T>(prev, curr, Hcur, B.x, B.pool, n, st, cells));
-      h->prof_end();
-      h->prof_begin(1);
-      LAUNCH(launch_conv_fused(B.fused, B.layers[1].out.p, make_geom(B.layers[1], n), n, num_sms, st));
-      for (size_t i = 2; i < nl; ++i)
-        if ((rc = run_conv<T>(h, B.layers[i], n))) return rc;
-      h->prof_end();
-      return UAHN_OK;
+  h->prof_begin(0);
+  LAUNCH(launch_warp_concat_pool<T>(prev, curr, Hcur, B.x, B.pool, n, st, cells));
+  h->prof_end();
+  h->prof_begin(1);
+  size_t first = 0;
+  if constexpr (sizeof(T) == 2) {
+    if (B.fused.enabled) {
+      LAUNCH(launch_conv_fused(B.fused, B.layers[1].out.p, make_geom(B.layers[1], n), n, h->num_sms, st));
+      first = 2;
     }
   }
-  for (int c0 = 0; c0 < n; c0 += CH) {
-    const int nc = std::min(CH, n - c0);
-    h->prof_begin(0);
-    LAUNCH(launch_warp_concat_pool<T>(prev + (size_t)c0 * IMG_PIXELS, curr + (size_t)c0 * IMG_PIXELS,
-                                      Hcur ? Hcur + (size_t)c0 * 9 : nullptr, B.x, B.pool, nc, st, CH >= n ? cells : nullptr));
-    h->prof_end();
-    h->prof_begin(1);
-    if ((rc = run_conv<T>(h, B.layers[0], nc))) return rc;
-    if (CH < h->cap && nl > 1 && (rc = run_conv<T>(h, B.layers[1], nc, (size_t)c0))) return rc;
-    h->prof_end();
-  }
-  h->prof_begin(1);
-  for (size_t i = (CH < h->cap ? 2 : 1); i < nl; ++i)
+  for (size_t i = first; i < nl; ++i)
     if ((rc = run_conv<T>(h, B.layers[i], n))) return rc;
   h->prof_end();
   return UAHN_OK;
@@ -484,7 +454,7 @@ int forward(uahn_handle* h, int n, const uint8_t* prev, const uint8_t* curr, con
   const int variant = h->cfg.variant;
   const float* Hcur = nullptr;
   int rc;
-  pdl_select(n);
+  g_pdl_on = true;
   if (variant != UAHN_VARIANT_FULL) {
     if (!prior) return h->fail(UAHN_ERR_INVALID, "this variant needs a prior");
     h->prof_begin(3);
@@ -595,7 +565,6 @@ int uahn_create(const uahn_config* cfg, uahn_handle** out) {
   h->cfg = *cfg;
   h->cap = cfg->max_batch;
   h->bf16 = cfg->precision == UAHN_PRECISION_BF16;
-  if (const char* e = getenv("UAHN_L2_CHUNK")) h->l2_chunk = std::max(1, atoi(e));
   h->es = h->bf16 ? 2 : 4;
   auto bail = [&](int rc) {
     g_create_error = h->last_error;
@@ -1193,7 +1162,8 @@ long uahn_debug_read(uahn_handle* h, const char* what, float* out, size_t capaci
         if (h->blocks[b].active && w.substr(4) == L.spec.name) t = &L.out;
   }
   if (!t) return h->fail(UAHN_ERR_INVALID, "unknown debug tensor '%s'", what);
-  if (n > t->N) return h->fail(UAHN_ERR_STATE, "'%s' is chunk-resident (%d pairs); rerun with n <= %d to read it", what, t->N, t->N);
+  // the fused fronts of blocks 3 and 4 never write conv 0's output: its buffer holds only what uahn_stage_conv put there
+  if (n > t->N) return h->fail(UAHN_ERR_STATE, "'%s' holds %d pairs; rerun with n <= %d to read it", what, t->N, t->N);
   const size_t count = (size_t)n * t->C * t->H * t->W;
   if (count > capacity) return h->fail(UAHN_ERR_INVALID, "capacity too small (%zu needed)", count);
   std::vector<uint8_t> raw((size_t)n * t->pitch_n * h->es);

@@ -1,12 +1,9 @@
 // Regression / uncertainty head kernels of the UAHN cascade:
-//   * 4-point DLT solve (model_to_trace.py:42-61): one warp per pair, Gauss-Jordan with partial pivoting,
-//     rows held one-per-lane, pivot search and row broadcast by warp shuffles, fp64 accumulation
+//   * 4-point DLT solve (model_to_trace.py:42-61) in closed form, fp64, every lane of a pair's warp redundantly
 //   * Linear(5120->8) + DLT + homography composition H <- H·H_b (model_to_trace.py:143-150,163-168,183-188)
 //   * MC-dropout expansion of the block-4 feature (model_to_trace.py:222-235,272-273)
 //   * second head layer, 16-sample ensemble (model_to_trace.py:274-281), covariance transfer
 //     (model_to_trace.py:18-38), output packing and the showError homography (model_to_trace.py:311-323)
-#include <cstdlib>
-
 #include "common.cuh"
 #include "kernels.h"
 #include "tc_ptx.cuh"
@@ -19,66 +16,15 @@ __device__ __forceinline__ void corner(int i, float& x, float& y) {   // model_t
   y = (i == 1 || i == 2) ? (float)(IMG_H - 1) : 0.f;
 }
 
-// All 32 lanes call with the same `dst` (4 destination points, fp32 like the reference's `pts0 + d`).
-// Lane r (mod 8) owns row r of the 8x9 augmented system; result h[0..8] (h[8] = 1) on every lane.
-// The general solver: Gauss-Jordan with partial pivoting by warp shuffles.  Since the latency work of round 2 the product path
-// takes dlt_rect below (the system always has the same four source points); UAHN_DLT_ELIMINATION=1 switches back.
-__device__ void dlt_elimination_warp(const float* dst, double* h) {
-  const int lane = threadIdx.x & 31, r = lane & 7, pt = r >> 1;
-  float sx, sy;
-  corner(pt, sx, sy);
-  const double x = sx, y = sy, u = dst[2 * pt], v = dst[2 * pt + 1];
-  double a[9];
-  if ((r & 1) == 0) {
-    a[0] = x; a[1] = y; a[2] = 1; a[3] = 0; a[4] = 0; a[5] = 0; a[6] = -u * x; a[7] = -u * y; a[8] = u;
-  } else {
-    a[0] = 0; a[1] = 0; a[2] = 0; a[3] = x; a[4] = y; a[5] = 1; a[6] = -v * x; a[7] = -v * y; a[8] = v;
-  }
-  bool used = false;
-  int mycol = -1;
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    double best = used ? -1.0 : fabs(a[c]);
-    int bi = r;
-#pragma unroll
-    for (int off = 4; off >= 1; off >>= 1) {
-      const double ov = __shfl_xor_sync(0xffffffffu, best, off, 8);
-      const int oi = __shfl_xor_sync(0xffffffffu, bi, off, 8);
-      if (ov > best || (ov == best && oi < bi)) { best = ov; bi = oi; }
-    }
-    const int p = bi;
-    const double piv = __shfl_sync(0xffffffffu, a[c], p, 8);
-    const double f = a[c] / piv;
-#pragma unroll
-    for (int j = c; j < 9; ++j) {
-      const double pj = __shfl_sync(0xffffffffu, a[j], p, 8);
-      if (r != p) a[j] -= f * pj;
-    }
-    if (r == p) { used = true; mycol = c; }
-  }
-  double diag = 1.0;
-#pragma unroll
-  for (int c = 0; c < 8; ++c)
-    if (mycol == c) diag = a[c];
-  const double xr = a[8] / diag;
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    const unsigned m = __ballot_sync(0xffffffffu, mycol == c && lane < 8);
-    const int owner = m ? (__ffs(m) - 1) : 0;
-    h[c] = __shfl_sync(0xffffffffu, xr, owner);
-  }
-  h[8] = 1.0;
-}
-
-// The same solve in closed form.  The four source points are always the corners of the 320 x 224 frame
+// The DLT solve.  The four source points are always the corners of the 320 x 224 frame
 // (model_to_trace.py:78-83), so the 8x8 system is the square-to-quadrilateral mapping (Heckbert, "Fundamentals of Texture
 // Mapping and Image Warping", 1989, sec. 2.2.3) composed with the frame's scaling: with (u, v) = (x / (W-1), y / (H-1)) and
 // the unit square's corners (0,0), (1,0), (1,1), (0,1) going to q0, q1, q2, q3,
 //   g = | S  d2 | / | d1 d2 |,  h = | d1 S | / | d1 d2 |   (d1 = q1 - q2, d2 = q3 - q2, S = q0 - q1 + q2 - q3),
 //   X = (a u + b v + c) / (g u + h v + 1) with a = q1.x - q0.x + g q1.x, b = q3.x - q0.x + h q3.x, c = q0.x (Y alike).
-// ~40 fp64 operations per lane and no shuffles instead of eight dependent elimination steps (~3 us of every DLT launch on the
-// batch-1 chain).  Same exact solution: in fp64 the two agree to ~1e-12, far inside the fp32 noise of the reference's
-// torch.inverse (tests/test_gpu_parity.py::test_stage_dlt_matches_reference runs both).
+// ~40 fp64 operations per lane and no shuffles: a warp-shuffle Gauss-Jordan elimination of the general system spends ~3 us
+// more per DLT launch on the batch-1 chain.  Same exact solution, far inside the fp32 noise of the reference's torch.inverse
+// (tests/test_gpu_parity.py::test_stage_dlt_matches_reference).
 __device__ __forceinline__ void dlt_rect(const float* dst, double* h) {
   // corner order of the model: UL, BL, BR, UR  ->  q0 = UL, q1 = UR, q2 = BR, q3 = BL
   const double x0 = dst[0], y0 = dst[1], x3 = dst[2], y3 = dst[3], x2 = dst[4], y2 = dst[5], x1 = dst[6], y1 = dst[7];
@@ -91,11 +37,6 @@ __device__ __forceinline__ void dlt_rect(const float* dst, double* h) {
   h[3] = ((y1 - y0) + g * y1) * IW; h[4] = ((y3 - y0) + k * y3) * IH; h[5] = y0;
   h[6] = g * IW; h[7] = k * IH; h[8] = 1.0;
 }
-__constant__ int c_dlt_elimination;      // 1: the warp-shuffle elimination (set once per process from UAHN_DLT_ELIMINATION)
-__device__ __forceinline__ void dlt_warp(const float* dst, double* h) {
-  if (c_dlt_elimination) dlt_elimination_warp(dst, h);
-  else dlt_rect(dst, h);
-}
 
 // fp32 3x3 product, k accumulated sequentially with FMA (torch.bmm on CPU)
 __device__ __forceinline__ void mat3_mul(const float* A, const float* B, float* C) {
@@ -106,22 +47,19 @@ __device__ __forceinline__ void mat3_mul(const float* A, const float* B, float* 
       C[i * 3 + j] = __fmaf_rn(A[i * 3 + 2], B[6 + j], __fmaf_rn(A[i * 3 + 1], B[3 + j], __fmul_rn(A[i * 3], B[j])));
 }
 
-// H = DLT(pts0, pts0 + off); optional left-multiplication by Hprev.  One warp per pair.
-__global__ void dlt_kernel(int n, const float* __restrict__ off, const float* __restrict__ Hprev, float* __restrict__ Hout) {
-  pdl_wait();
-  pdl_launch_dependents();
-  const int pair = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  if (pair >= n) return;
+// The tail of every DLT-bearing stage, for the 8 offsets d of one pair: H_b = DLT(pts0, pts0 + d), then
+// Hout[pair] = Hprev ? Hprev[pair]·H_b : H_b.  Called by a whole warp: every lane solves, lane 0 stores.
+__device__ __forceinline__ void dlt_compose_store(const float* d, int pair, const float* Hprev, float* Hout) {
   float dst[8];
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     float x, y;
     corner(i, x, y);
-    dst[2 * i] = __fadd_rn(x, off[pair * 8 + 2 * i]);
-    dst[2 * i + 1] = __fadd_rn(y, off[pair * 8 + 2 * i + 1]);
+    dst[2 * i] = __fadd_rn(x, d[2 * i]);
+    dst[2 * i + 1] = __fadd_rn(y, d[2 * i + 1]);
   }
   double h[9];
-  dlt_warp(dst, h);
+  dlt_rect(dst, h);
   if ((threadIdx.x & 31) == 0) {
     float hb[9], out[9];
 #pragma unroll
@@ -140,91 +78,20 @@ __global__ void dlt_kernel(int n, const float* __restrict__ off, const float* __
   }
 }
 
-// d = W8·feat + b8 ; H_b = DLT(pts0, pts0 + d) ; Hout = Hprev ? Hprev·H_b : H_b.
-// FC8_PAIRS pairs per CTA so each 8x5120 weight read from L2 is shared by 4 feature vectors.
-// feat is the last conv output in NHWC order ((h*5+w)*256 + c); W8 was permuted to that order at load.
-constexpr int FC8_PAIRS = 4;
-constexpr int FC8_SMALL_MAX = 8;   // up to here: fc8_dlt_cluster_kernel (split-K over a cluster)
-template <typename T>
-__global__ void __launch_bounds__(256) fc8_dlt_kernel(int n, const T* __restrict__ feat, const float* __restrict__ W8,
-                                                       const float* __restrict__ b8, const float* __restrict__ Hprev,
-                                                       float* __restrict__ Hout, float* __restrict__ dout) {
+// H = DLT(pts0, pts0 + off); optional left-multiplication by Hprev.  One warp per pair.
+__global__ void dlt_kernel(int n, const float* __restrict__ off, const float* __restrict__ Hprev, float* __restrict__ Hout) {
   pdl_wait();
   pdl_launch_dependents();
-  __shared__ float part[8][FC8_PAIRS][8];
-  __shared__ float d_s[FC8_PAIRS][8];
-  const int pair0 = blockIdx.x * FC8_PAIRS, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  const int np = min(FC8_PAIRS, n - pair0);
-  float acc[FC8_PAIRS][8];
-#pragma unroll
-  for (int p = 0; p < FC8_PAIRS; ++p)
-#pragma unroll
-    for (int o = 0; o < 8; ++o) acc[p][o] = 0.f;
-#pragma unroll 5        // 20 trips; 5 x (8 weight + np feature) loads in flight per thread: the loop is L2-latency-bound
-  for (int k = tid; k < FC_IN; k += 256) {
-    float w[8], x[FC8_PAIRS];
-#pragma unroll
-    for (int o = 0; o < 8; ++o) w[o] = __ldg(W8 + o * FC_IN + k);
-#pragma unroll
-    for (int p = 0; p < FC8_PAIRS; ++p) x[p] = p < np ? to_f32<T>(feat[(size_t)(pair0 + p) * FC_IN + k]) : 0.f;
-#pragma unroll
-    for (int p = 0; p < FC8_PAIRS; ++p)
-#pragma unroll
-      for (int o = 0; o < 8; ++o) acc[p][o] = fmaf(x[p], w[o], acc[p][o]);
-  }
-#pragma unroll
-  for (int p = 0; p < FC8_PAIRS; ++p)
-#pragma unroll
-    for (int o = 0; o < 8; ++o) {
-#pragma unroll
-      for (int s = 16; s >= 1; s >>= 1) acc[p][o] += __shfl_xor_sync(0xffffffffu, acc[p][o], s);
-      if (lane == 0) part[wid][p][o] = acc[p][o];
-    }
-  __syncthreads();
-  if (tid < FC8_PAIRS * 8) {
-    const int p = tid >> 3, o = tid & 7;
-    float s = 0.f;
-#pragma unroll
-    for (int w = 0; w < 8; ++w) s += part[w][p][o];
-    s += b8[o];
-    d_s[p][o] = s;
-    if (dout && p < np) dout[(pair0 + p) * 8 + o] = s;
-  }
-  __syncthreads();
-  if (wid < np) {                       // one warp per pair: DLT + composition
-    const int pair = pair0 + wid;
-    float dst[8];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      float x, y;
-      corner(i, x, y);
-      dst[2 * i] = __fadd_rn(x, d_s[wid][2 * i]);
-      dst[2 * i + 1] = __fadd_rn(y, d_s[wid][2 * i + 1]);
-    }
-    double h[9];
-    dlt_warp(dst, h);
-    if (lane == 0) {
-      float hb[9], out[9];
-#pragma unroll
-      for (int i = 0; i < 9; ++i) hb[i] = (float)h[i];
-      if (Hprev) {
-        float hp[9];
-#pragma unroll
-        for (int i = 0; i < 9; ++i) hp[i] = Hprev[pair * 9 + i];
-        mat3_mul(hp, hb, out);
-      } else {
-#pragma unroll
-        for (int i = 0; i < 9; ++i) out[i] = hb[i];
-      }
-#pragma unroll
-      for (int i = 0; i < 9; ++i) Hout[pair * 9 + i] = out[i];
-    }
-  }
+  const int pair = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (pair >= n) return;
+  dlt_compose_store(off + pair * 8, pair, Hprev, Hout);
 }
 
+// d = W8·feat + b8 ; H_b = DLT(pts0, pts0 + d) ; Hout = Hprev ? Hprev·H_b : H_b.
+// feat is the last conv output in NHWC order ((h*5+w)*256 + c); W8 was permuted to that order at load.
 // Batch path (round 2): eight pairs per CTA.  A thread owns five 4-element slices of k (k = 4 (t + 256 i)): per slice eight
-// 16-byte weight loads serve 8 pairs x 8 outputs x 4 k = 256 FMAs, so the L2 -> SM weight traffic per pair halves against
-// fc8_dlt_kernel (4 pairs per CTA, scalar loads) and a thread waits for 5 batches of 16 wide loads instead of 20 trips of 12
+// 16-byte weight loads serve 8 pairs x 8 outputs x 4 k = 256 FMAs, so the L2 -> SM weight traffic per pair is half that of
+// 4 pairs per CTA with scalar loads, and a thread waits for 5 batches of 16 wide loads instead of 20 trips of 12
 // scalar ones — the stage is a chain of L2 round trips, nothing else (16 us per launch at 1024 pairs, issue slots 23 % busy).
 // The 64 partial sums of a thread meet in shared memory ([output][thread], conflict-free) and are added in a fixed order.
 constexpr int FC8W_PAIRS = 8;
@@ -237,7 +104,7 @@ __global__ void __launch_bounds__(256, 1) fc8_dlt_wide_kernel(int n, const T* __
   pdl_launch_dependents();
   extern __shared__ __align__(16) float red_w[];              // [64][257]
   __shared__ float d_s[FC8W_PAIRS][8];
-  const int pair0 = blockIdx.x * FC8W_PAIRS, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+  const int pair0 = blockIdx.x * FC8W_PAIRS, tid = threadIdx.x, wid = tid >> 5;
   const int np = min(FC8W_PAIRS, n - pair0);
   float acc[FC8W_PAIRS][8];
 #pragma unroll
@@ -291,40 +158,13 @@ __global__ void __launch_bounds__(256, 1) fc8_dlt_wide_kernel(int n, const T* __
     }
   }
   __syncthreads();
-  if (wid < np) {                       // one warp per pair: DLT + composition
-    const int pair = pair0 + wid;
-    float dst[8];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      float x, y;
-      corner(i, x, y);
-      dst[2 * i] = __fadd_rn(x, d_s[wid][2 * i]);
-      dst[2 * i + 1] = __fadd_rn(y, d_s[wid][2 * i + 1]);
-    }
-    double h[9];
-    dlt_warp(dst, h);
-    if (lane == 0) {
-      float hb[9], out[9];
-#pragma unroll
-      for (int i = 0; i < 9; ++i) hb[i] = (float)h[i];
-      if (Hprev) {
-        float hp[9];
-#pragma unroll
-        for (int i = 0; i < 9; ++i) hp[i] = Hprev[pair * 9 + i];
-        mat3_mul(hp, hb, out);
-      } else {
-#pragma unroll
-        for (int i = 0; i < 9; ++i) out[i] = hb[i];
-      }
-#pragma unroll
-      for (int i = 0; i < 9; ++i) Hout[pair * 9 + i] = out[i];
-    }
-  }
+  if (wid < np) dlt_compose_store(d_s[wid], pair0 + wid, Hprev, Hout);   // one warp per pair
 }
 
 // Latency path (<= FC8_SMALL_MAX pairs): the same stage with the 5120-long dot products split over a cluster of 8 CTAs per
 // pair (640 k each, 8 x fewer dependent L2 round trips per thread), partial sums reduced through distributed shared
 // memory into rank 0, which adds the bias and runs the DLT + composition.  (One CTA per 4 pairs takes 20 us at batch 1.)
+constexpr int FC8_SMALL_MAX = 8;
 constexpr int FC8_CLUSTER = 8;
 template <typename T>
 __global__ void __cluster_dims__(FC8_CLUSTER, 1, 1) __launch_bounds__(256)
@@ -389,34 +229,7 @@ __global__ void __cluster_dims__(FC8_CLUSTER, 1, 1) __launch_bounds__(256)
     if (dout) dout[pair * 8 + tid] = v;
   }
   __syncthreads();
-  if (wid == 0) {                            // one warp: DLT + composition
-    float dst[8];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      float x, y;
-      corner(i, x, y);
-      dst[2 * i] = __fadd_rn(x, d_s[2 * i]);
-      dst[2 * i + 1] = __fadd_rn(y, d_s[2 * i + 1]);
-    }
-    double h[9];
-    dlt_warp(dst, h);
-    if (lane == 0) {
-      float hb[9], out[9];
-#pragma unroll
-      for (int i = 0; i < 9; ++i) hb[i] = (float)h[i];
-      if (Hprev) {
-        float hp[9];
-#pragma unroll
-        for (int i = 0; i < 9; ++i) hp[i] = Hprev[pair * 9 + i];
-        mat3_mul(hp, hb, out);
-      } else {
-#pragma unroll
-        for (int i = 0; i < 9; ++i) out[i] = hb[i];
-      }
-#pragma unroll
-      for (int i = 0; i < 9; ++i) Hout[pair * 9 + i] = out[i];
-    }
-  }
+  if (wid == 0) dlt_compose_store(d_s, pair, Hprev, Hout);   // one warp
 }
 
 // A'[head][pair][s][k'] = keep ? feat[k'] * (1/0.95) : 0     (Dropout(0.05) on the repeated feature)
@@ -824,7 +637,7 @@ __global__ void __launch_bounds__(256) mc_final_kernel(const T* __restrict__ hid
                                  o.mean + pair * 8, o.cov + (size_t)pair * 64);
     if (o.Htot) {                                       // model_to_trace.py:321-323
       double h4[9];
-      dlt_warp(ptsw, h4);
+      dlt_rect(ptsw, h4);
       if (lane == 0) {
         float hb[9], out[9];
 #pragma unroll
@@ -855,9 +668,6 @@ cudaError_t launch_fc8_dlt(int n, const T* feat, const float* W8, const float* b
                            float* dout, cudaStream_t st) {
   if (n <= FC8_SMALL_MAX)   // latency path: a cluster of 8 CTAs per pair (compile-time cluster dimensions)
     return launch_pdl(fc8_dlt_cluster_kernel<T>, dim3(FC8_CLUSTER * n), dim3(256), 0, st, n, feat, W8, b8, Hprev, Hout, dout);
-  static const bool narrow = getenv("UAHN_FC8_NARROW") != nullptr;      // A/B: the 4-pairs-per-CTA kernel
-  if (narrow)
-    return launch_pdl(fc8_dlt_kernel<T>, dim3((n + FC8_PAIRS - 1) / FC8_PAIRS), dim3(256), 0, st, n, feat, W8, b8, Hprev, Hout, dout);
   static SmemOptIn optin;   // per device (common.cuh)
   if (cudaError_t e = optin.ensure(fc8_dlt_wide_kernel<T>, FC8W_SMEM); e != cudaSuccess) return e;
   return launch_pdl(fc8_dlt_wide_kernel<T>, dim3((n + FC8W_PAIRS - 1) / FC8W_PAIRS), dim3(256), FC8W_SMEM, st, n, feat, W8, b8, Hprev, Hout, dout);
@@ -892,8 +702,6 @@ cudaError_t launch_mc_fc1_small_fused(int n, const void* feat, const void* Wm, c
 
 // host side: build the alias table and upload it to the current device (idempotent; called by uahn_create)
 cudaError_t init_keep_alias_table() {
-  const int elim = getenv("UAHN_DLT_ELIMINATION") != nullptr;   // (rides along: both are per-device constants set at create)
-  if (cudaError_t e = cudaMemcpyToSymbol(c_dlt_elimination, &elim, sizeof(elim)); e != cudaSuccess) return e;
   uint32_t tab[256];
   build_keep_alias_table(tab);
   return cudaMemcpyToSymbol(g_keep_alias, tab, sizeof(tab));
