@@ -25,6 +25,9 @@ EXPORTED_SYMBOLS = [
 PREPROC_SYMBOLS = ["uahn_undistort_init_maps", "uahn_set_undistort_maps", "uahn_load_raw_image", "uahn_stage_undistort"]
 EKF_SYMBOLS = ["uahn_ekf_prior_px", "uahn_ekf_update", "uahn_ekf_reset_offsets", "uahn_ekf_iekf_frame",
                "uahn_imu_select_readings", "uahn_imu_predict_and_compute", "uahn_imu_propagate"]
+FILTER_SYMBOLS = ["uahn_filter_create", "uahn_filter_destroy", "uahn_filter_set_states", "uahn_filter_get_states",
+                  "uahn_filter_propagate", "uahn_filter_frame", "uahn_filter_wait"]
+ERR_INVALID, ERR_STATE, ERR_UNSUPPORTED = -1, -4, -5
 
 
 class UahnError(RuntimeError):
@@ -201,6 +204,19 @@ def load_library(path: str | None = None):
     lib.uahn_imu_predict_and_compute.restype = i
     lib.uahn_imu_propagate.argtypes = [vp, ekf, vp, i, dbl, dbl, vp]
     lib.uahn_imu_propagate.restype = i
+    lib.uahn_filter_create.argtypes = [vp, i, vp, C.POINTER(vp)]
+    lib.uahn_filter_create.restype = i
+    lib.uahn_filter_destroy.argtypes = [vp]
+    lib.uahn_filter_destroy.restype = None
+    for f in (lib.uahn_filter_set_states, lib.uahn_filter_get_states):
+        f.argtypes = [vp, i, i, vp]
+        f.restype = i
+    lib.uahn_filter_propagate.argtypes = [vp, vp, vp, vp, vp]
+    lib.uahn_filter_propagate.restype = i
+    lib.uahn_filter_frame.argtypes = [vp, vp, vp, i, dbl, i, vp, C.POINTER(_Rng), vp, vp, vp, vp]
+    lib.uahn_filter_frame.restype = i
+    lib.uahn_filter_wait.argtypes = [vp, vp]
+    lib.uahn_filter_wait.restype = i
     if path is None:
         _lib = lib
     return lib
@@ -509,3 +525,87 @@ class HomographyNet:
 
     def get_latest_inference_time(self) -> float:
         return self._main.latest_inference_time
+
+
+class FilterBank:
+    """n EKF states on the device next to one Uahn handle (include/uahn_filter.h).
+
+    States are numpy arrays: imu [k, 16], offsets [k, 4, 3], cov [k, 27, 27] (float64).  propagate() and frame() only
+    enqueue work; their inputs must stay alive and their outputs are valid once wait() has returned."""
+
+    def __init__(self, net: "Uahn", n: int, cfg: "PropagatorConfig"):
+        self._lib, self.net, self.n = net._lib, net, n
+        self._f = C.c_void_p()
+        self._cfg = cfg
+        self._keep = []
+        net._check(self._lib.uahn_filter_create(net._h, n, C.byref(cfg), C.byref(self._f)))
+
+    def close(self):
+        f = getattr(self, "_f", None)
+        if f is not None and f.value:
+            self._lib.uahn_filter_destroy(f)
+            self._f = None
+
+    __del__ = close
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    def _check(self, rc):
+        return self.net._check(rc)
+
+    def set_states(self, first: int, imu, offsets, cov):
+        imu = np.asarray(imu, np.float64).reshape(-1, 16)
+        k = imu.shape[0]
+        raw = np.empty((k, 16 + 12 + 27 * 27), np.float64)      # uahn_ekf_state rows
+        raw[:, :16] = imu
+        raw[:, 16:28] = np.asarray(offsets, np.float64).reshape(k, 12)
+        raw[:, 28:] = np.asarray(cov, np.float64).reshape(k, 27 * 27)
+        self._check(self._lib.uahn_filter_set_states(self._f, first, k, _ptr(raw)))
+
+    def get_states(self, first: int = 0, count: int | None = None):
+        """→ (imu [k, 16], offsets [k, 4, 3], cov [k, 27, 27])"""
+        count = self.n - first if count is None else count
+        raw = np.empty((count, 16 + 12 + 27 * 27), np.float64)
+        self._check(self._lib.uahn_filter_get_states(self._f, first, count, _ptr(raw)))
+        return raw[:, :16].copy(), raw[:, 16:28].reshape(count, 4, 3).copy(), raw[:, 28:].reshape(count, 27, 27).copy()
+
+    def propagate(self, readings, t0, t1):
+        """readings: one list of (t, wm[3], am[3]) per slot; t0 / t1: per-slot interval ends."""
+        flat = [r for slot in readings for r in slot]
+        offsets = np.zeros(self.n + 1, np.int32)
+        offsets[1:] = np.cumsum([len(slot) for slot in readings])
+        imu = _imu_array(flat) if flat else (ImuSample * 1)()
+        t0, t1 = np.ascontiguousarray(t0, np.float64), np.ascontiguousarray(t1, np.float64)
+        self._keep += [imu, offsets, t0, t1]
+        self._check(self._lib.uahn_filter_propagate(self._f, imu, _ptr(offsets), _ptr(t0), _ptr(t1)))
+
+    def frame(self, frames, max_iter: int = 1, K_net_Cov: float = 10.0, min_images: int = 10, use_measurement=None,
+              seed: int = 0, first_pair: int | None = None, iterative: "Uahn | None" = None, keep_masks=None):
+        """One IEKF frame for every slot → dict of numpy outputs (prior/mean [max_iter, n, 8], cov [max_iter, n, 8, 8],
+        imu [n, 16]), filled when wait() returns.  first_pair None: the bank numbers its frames itself."""
+        frames = np.ascontiguousarray(frames, np.uint8)
+        assert frames.shape == (self.n, IMG_H, IMG_W)
+        use = None if use_measurement is None else np.ascontiguousarray(use_measurement, np.uint8)
+        out = {"prior": np.empty((max_iter, self.n, 8), np.float32), "mean": np.empty((max_iter, self.n, 8), np.float32),
+               "cov": np.empty((max_iter, self.n, 8, 8), np.float32), "imu": np.empty((self.n, 16), np.float64)}
+        rng = None
+        if first_pair is not None or seed or keep_masks is not None:
+            rng = C.byref(_Rng(seed, first_pair or 0, _ptr(keep_masks).value if keep_masks is not None else None))
+        self._keep += [frames, use, out]
+        self._check(self._lib.uahn_filter_frame(self._f, iterative._h if iterative else None, _ptr(frames), max_iter,
+                                                float(K_net_Cov), min_images, _ptr(use), rng, _ptr(out["prior"]),
+                                                _ptr(out["mean"]), _ptr(out["cov"]), _ptr(out["imu"])))
+        return out
+
+    def wait(self):
+        """→ per-slot codes since the previous wait (0, ERR_STATE, ERR_INVALID)."""
+        status = np.zeros(self.n, np.int32)
+        rc = self._lib.uahn_filter_wait(self._f, _ptr(status))
+        self._keep = []
+        if rc not in (0, ERR_STATE, ERR_INVALID):
+            self._check(rc)
+        return status

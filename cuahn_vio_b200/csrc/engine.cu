@@ -1187,3 +1187,10 @@ long uahn_debug_read(uahn_handle* h, const char* what, float* out, size_t capaci
 }
 
 }  // extern "C"
+
+// what the filter bank (filter_bank.cu) needs of a handle
+namespace uahn {
+int handle_device(const uahn_handle* h) { return h->cfg.device; }
+int handle_max_batch(const uahn_handle* h) { return h->cap; }
+int handle_fail(uahn_handle* h, int code, const char* msg) { return h->fail(code, "%s", msg); }
+}  // namespace uahn

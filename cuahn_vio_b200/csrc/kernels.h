@@ -2,7 +2,14 @@
 #pragma once
 #include "common.cuh"
 
+struct uahn_handle;
+
 namespace uahn {
+
+// engine.cu: what the filter bank (filter_bank.cu) needs of a handle; handle_fail records `msg` for uahn_last_error
+int handle_device(const uahn_handle* h);
+int handle_max_batch(const uahn_handle* h);
+int handle_fail(uahn_handle* h, int code, const char* msg);
 
 // image_kernels.cu
 // The current frames of one call as zero-separated cells of a 2-D CUDA array: the source of the texture-gather warp kernel
