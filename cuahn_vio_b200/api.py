@@ -26,7 +26,8 @@ PREPROC_SYMBOLS = ["uahn_undistort_init_maps", "uahn_set_undistort_maps", "uahn_
 EKF_SYMBOLS = ["uahn_ekf_prior_px", "uahn_ekf_update", "uahn_ekf_reset_offsets", "uahn_ekf_iekf_frame",
                "uahn_imu_select_readings", "uahn_imu_predict_and_compute", "uahn_imu_propagate"]
 FILTER_SYMBOLS = ["uahn_filter_create", "uahn_filter_destroy", "uahn_filter_set_states", "uahn_filter_get_states",
-                  "uahn_filter_propagate", "uahn_filter_frame", "uahn_filter_wait"]
+                  "uahn_filter_propagate", "uahn_filter_frame", "uahn_filter_wait", "uahn_filter_set_undistort_maps",
+                  "uahn_filter_frame_raw", "uahn_filter_stage_undistort"]
 ERR_INVALID, ERR_STATE, ERR_UNSUPPORTED = -1, -4, -5
 
 
@@ -217,6 +218,12 @@ def load_library(path: str | None = None):
     lib.uahn_filter_frame.restype = i
     lib.uahn_filter_wait.argtypes = [vp, vp]
     lib.uahn_filter_wait.restype = i
+    lib.uahn_filter_set_undistort_maps.argtypes = [vp, i, i, vp, vp]
+    lib.uahn_filter_set_undistort_maps.restype = i
+    lib.uahn_filter_frame_raw.argtypes = [vp, vp, vp, C.c_size_t, i, dbl, i, vp, C.POINTER(_Rng), vp, vp, vp, vp]
+    lib.uahn_filter_frame_raw.restype = i
+    lib.uahn_filter_stage_undistort.argtypes = [vp, vp, C.c_size_t, vp]
+    lib.uahn_filter_stage_undistort.restype = i
     if path is None:
         _lib = lib
     return lib
@@ -538,6 +545,7 @@ class FilterBank:
         self._f = C.c_void_p()
         self._cfg = cfg
         self._keep = []
+        self._raw_shape = None       # (raw_rows, raw_cols) of the maps set last
         net._check(self._lib.uahn_filter_create(net._h, n, C.byref(cfg), C.byref(self._f)))
 
     def close(self):
@@ -589,6 +597,19 @@ class FilterBank:
         imu [n, 16]), filled when wait() returns.  first_pair None: the bank numbers its frames itself."""
         frames = np.ascontiguousarray(frames, np.uint8)
         assert frames.shape == (self.n, IMG_H, IMG_W)
+        return self._frame(self._lib.uahn_filter_frame, (_ptr(frames),), frames, max_iter, K_net_Cov, min_images,
+                           use_measurement, seed, first_pair, iterative, keep_masks)
+
+    def frame_raw(self, raw, max_iter: int = 1, K_net_Cov: float = 10.0, min_images: int = 10, use_measurement=None,
+                  seed: int = 0, first_pair: int | None = None, iterative: "Uahn | None" = None, keep_masks=None):
+        """frame() with raw camera frames [n, raw_rows, raw_cols] u8 (any row stride), undistorted on the device with the
+        maps of set_undistort_maps(); same arguments and outputs as frame()."""
+        raw, stride = self._raw_frames(raw)
+        return self._frame(self._lib.uahn_filter_frame_raw, (_ptr(raw), stride), raw, max_iter, K_net_Cov, min_images,
+                           use_measurement, seed, first_pair, iterative, keep_masks)
+
+    def _frame(self, fn, frame_args, frames, max_iter, K_net_Cov, min_images, use_measurement, seed, first_pair, iterative,
+               keep_masks):
         use = None if use_measurement is None else np.ascontiguousarray(use_measurement, np.uint8)
         out = {"prior": np.empty((max_iter, self.n, 8), np.float32), "mean": np.empty((max_iter, self.n, 8), np.float32),
                "cov": np.empty((max_iter, self.n, 8, 8), np.float32), "imu": np.empty((self.n, 16), np.float64)}
@@ -596,10 +617,37 @@ class FilterBank:
         if first_pair is not None or seed or keep_masks is not None:
             rng = C.byref(_Rng(seed, first_pair or 0, _ptr(keep_masks).value if keep_masks is not None else None))
         self._keep += [frames, use, out]
-        self._check(self._lib.uahn_filter_frame(self._f, iterative._h if iterative else None, _ptr(frames), max_iter,
-                                                float(K_net_Cov), min_images, _ptr(use), rng, _ptr(out["prior"]),
-                                                _ptr(out["mean"]), _ptr(out["cov"]), _ptr(out["imu"])))
+        self._check(fn(self._f, iterative._h if iterative else None, *frame_args, max_iter, float(K_net_Cov), min_images,
+                       _ptr(use), rng, _ptr(out["prior"]), _ptr(out["mean"]), _ptr(out["cov"]), _ptr(out["imu"])))
         return out
+
+    def set_undistort_maps(self, raw_rows: int, raw_cols: int, map1: np.ndarray, map2: np.ndarray):
+        """One camera for every slot: map1 / map2 float32 [224, 320] (undistort_init_maps), raw frames raw_rows x raw_cols."""
+        m1, m2 = np.ascontiguousarray(map1, np.float32), np.ascontiguousarray(map2, np.float32)
+        assert m1.shape == (IMG_H, IMG_W) and m2.shape == (IMG_H, IMG_W)
+        self._raw_shape = None
+        self._check(self._lib.uahn_filter_set_undistort_maps(self._f, raw_rows, raw_cols, _ptr(m1), _ptr(m2)))
+        self._raw_shape = (raw_rows, raw_cols)
+
+    def stage_undistort(self, raw) -> np.ndarray:
+        """The n raw frames [n, raw_rows, raw_cols] remapped with the bank's maps → [n, 224, 320] u8 (synchronous)."""
+        raw, stride = self._raw_frames(raw)
+        out = np.empty((self.n, IMG_H, IMG_W), np.uint8)
+        self._check(self._lib.uahn_filter_stage_undistort(self._f, _ptr(raw), stride, _ptr(out)))
+        return out
+
+    def _raw_frames(self, raw):
+        """→ (array, row stride): [n, rows, cols] u8 whose frames sit rows * stride bytes apart, copied only if they do not."""
+        raw = np.asarray(raw)
+        assert raw.dtype == np.uint8 and raw.ndim == 3 and raw.shape[0] == self.n, (raw.dtype, raw.shape)
+        rows, cols = raw.shape[1:]
+        # the library reads rows x cols of the maps' raw size: a smaller array would be read past its end
+        assert self._raw_shape is None or (rows, cols) == self._raw_shape, ((rows, cols), self._raw_shape)
+        s0, s1, s2 = raw.strides
+        if not (s2 == 1 and s1 >= cols and (self.n == 1 or s0 == rows * s1)):
+            raw = np.ascontiguousarray(raw)
+            s1 = cols
+        return raw, s1
 
     def wait(self):
         """→ per-slot codes since the previous wait (0, ERR_STATE, ERR_INVALID)."""

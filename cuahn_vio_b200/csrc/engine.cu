@@ -961,7 +961,7 @@ int stage_raw(uahn_handle* h, const uint8_t* raw, int rows, int cols, size_t str
   CK(cudaStreamSynchronize(h->stream));   // h_raw may still be in flight from the previous frame
   for (int y = 0; y < rows; ++y) memcpy(h->h_raw + (size_t)y * cols, raw + (size_t)y * stride, cols);
   CK(cudaMemcpyAsync(h->d_raw, h->h_raw, (size_t)rows * cols, cudaMemcpyHostToDevice, h->stream));
-  LAUNCH(launch_remap_u8(h->d_raw, rows, cols, h->d_map1, h->d_map2, d_out, h->stream));
+  LAUNCH(launch_remap_u8(h->d_raw, rows, cols, (size_t)cols, 1, h->d_map1, h->d_map2, d_out, h->stream));
   return UAHN_OK;
 }
 }  // namespace

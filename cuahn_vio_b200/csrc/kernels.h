@@ -34,9 +34,10 @@ cudaError_t launch_warp_concat_pool(const uint8_t* prev, const uint8_t* curr, co
 cudaError_t launch_warp_plain(const uint8_t* prev, const uint8_t* curr, const float* Hmat, float* out, uint8_t* out_u8,
                               int16_t* ix, int16_t* iy, int error_map, int n, cudaStream_t st, int allow_fast);
 
-// cv::remap(INTER_LINEAR, constant-0 border) of a raw u8 frame through float maps into a 224x320 u8 image
-cudaError_t launch_remap_u8(const uint8_t* raw, int rows, int cols, const float* map1, const float* map2, uint8_t* out,
-                            cudaStream_t st);
+// cv::remap(INTER_LINEAR, constant-0 border) of n raw u8 frames through one pair of float maps (224x320 each) into n
+// 224x320 u8 images.  Raw frame i's row y starts at raw + (i * rows + y) * pitch; out is [n][224][320].
+cudaError_t launch_remap_u8(const uint8_t* raw, int rows, int cols, size_t pitch, int n, const float* map1,
+                            const float* map2, uint8_t* out, cudaStream_t st);
 
 // conv_f32.cu
 // ws: optional split-K workspace (ws_floats floats) for the small-M deep layers of the latency path; rows_per_pair: GEMM rows

@@ -7,7 +7,8 @@
  * network (uahn_ekf_iekf_frame).  Per slot the result is what uahn_imu_propagate / uahn_ekf_iekf_frame leave in that
  * slot's uahn_ekf_state (fp64 on both sides; see DESIGN §11 for how close).
  *
- * Asynchronous calls: uahn_filter_propagate and uahn_filter_frame only enqueue work on the stream of the bank's handle.
+ * Asynchronous calls: uahn_filter_propagate, uahn_filter_frame and uahn_filter_frame_raw only enqueue work on the stream
+ * of the bank's handle (and, for raw frames, on the bank's copy stream).
  * Their HOST inputs are borrowed until uahn_filter_wait returns, and their HOST outputs land there (the contract of
  * uahn_submit_batch / uahn_wait; pinned buffers are recommended).  Messages of failed calls: uahn_last_error(h).
  */
@@ -54,6 +55,26 @@ UAHN_API int uahn_filter_propagate(uahn_filter* f, const uahn_imu_sample* imu, c
 UAHN_API int uahn_filter_frame(uahn_filter* f, uahn_handle* h_iter, const uint8_t* frames, int max_iter, double K_net_Cov,
                                int min_images, const uint8_t* use_measurement, const uahn_rng* rng, float* prior_out,
                                float* mean_out, float* cov_out, double* imu_out);
+
+/* Raw camera frames (undistort + resize on the device, as uahn_set_undistort_maps / uahn_load_raw_image do for one
+ * handle).  One camera per bank (the bank already has one propagator config, i.e. one rig).  map1 / map2: HOST, 224*320
+ * floats each (uahn_undistort_init_maps' output); raw frames are raw_rows x raw_cols u8 (2 ... 32767 each).  Allocates the
+ * raw staging (2 x n raw frames on the device) and the bank's copy stream on first use; synchronous. */
+UAHN_API int uahn_filter_set_undistort_maps(uahn_filter* f, int raw_rows, int raw_cols, const float* map1, const float* map2);
+
+/* uahn_filter_frame with raw frames: raw holds n HOST frames [n][raw_rows][stride] (stride >= raw_cols bytes, slot i's
+ * frame at raw + i * raw_rows * stride).  Slot i's current frame becomes remap(raw_i) (cv::remap INTER_LINEAR,
+ * constant-0 border, bit for bit); everything after that (ring flip, priors, forwards, updates, outputs, rng numbering,
+ * status) is exactly uahn_filter_frame's, and the two calls may alternate on one bank.  The upload runs on the bank's copy
+ * stream into one of two staging buffers, so with pinned frames the upload of the next call overlaps this call's
+ * forward.  UAHN_ERR_STATE without maps. */
+UAHN_API int uahn_filter_frame_raw(uahn_filter* f, uahn_handle* h_iter, const uint8_t* raw, size_t stride, int max_iter,
+                                   double K_net_Cov, int min_images, const uint8_t* use_measurement, const uahn_rng* rng,
+                                   float* prior_out, float* mean_out, float* cov_out, double* imu_out);
+
+/* Parity entry, in the manner of uahn_stage_undistort: remap n raw frames (laid out as for uahn_filter_frame_raw) with
+ * the bank's maps into out (HOST, n x 224 x 320 u8) without touching the bank's ring or states; synchronous. */
+UAHN_API int uahn_filter_stage_undistort(uahn_filter* f, const uint8_t* raw, size_t stride, uint8_t* out);
 
 /* Waits for everything enqueued on the bank; status (optional): n per-slot codes since the previous wait (UAHN_OK,
  * UAHN_ERR_STATE, UAHN_ERR_INVALID).  Returns the first nonzero slot code, else UAHN_OK (or a CUDA error). */

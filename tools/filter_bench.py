@@ -8,7 +8,15 @@ arms, timed in the same process and alternated:
 The bank's filter-kernel time per step comes from CUDA kernel records of torch.profiler in a separate pass.  Frames and
 IMU readings are generated from seeds before timing.  Prints one JSON line; --out FILE also writes it to FILE.
 
-  python tools/filter_bench.py [--sizes 128 1024] [--frames 64] [--host-steps 4] [--out FILE]
+--raw adds, per size, two arms alternated with the bank arm, and a "raw" record:
+  raw bank  uahn_filter_propagate + uahn_filter_frame_raw per step: pinned 640x480 frames (synthetic_raw_frame, a few
+            unique ones tiled to S) undistorted on the device with the uahn_undistort_init_maps maps of one fixture camera
+  ceiling   a bare pinned cudaMemcpyAsync of the same raw bytes per step
+A profiled raw-bank pass of its own gives the remap kernel's and the filter kernels' time per step, the device time of the
+host-to-device copies and how much of it ran while a kernel was running.  raw_step_over_bound = raw-bank step /
+max(ceiling copy time, network step + filter kernels + remap), every term from the same run.
+
+  python tools/filter_bench.py [--sizes 128 1024] [--frames 64] [--host-steps 4] [--raw] [--out FILE]
 """
 from __future__ import annotations
 
@@ -29,6 +37,9 @@ HZ_IMU, HZ_CAM = 500.0, 30.0
 # filters from diverging over the timed frames (the work per update does not depend on it)
 K_NET_COV = 1000.0
 IMU_DTYPE = np.dtype([("t", np.float64), ("wm", np.float64, 3), ("am", np.float64, 3)])   # uahn_imu_sample
+RAW_ROWS, RAW_COLS, RAW_UNIQUE = 480, 640, 8
+RAW_CAMERA = "uzhfpv_indoor_fwd"                 # a fisheye camera of tests/golden/preproc.npz
+HBM_BYTES_PER_S = 7.7e12                         # B200 data sheet (one GPU): the bound the remap kernel is held to
 
 
 def gpu_info():
@@ -73,7 +84,7 @@ def pinned(shape, dtype):
     return torch.empty(shape, dtype=dtype, pin_memory=True).numpy()
 
 
-def run_size(api, wfile, S, n_frames, host_steps, rounds):
+def run_size(api, wfile, S, n_frames, host_steps, rounds, raw_arms=False):
     import torch
     lib = api.load_library()
     rng = np.random.default_rng(S)
@@ -155,20 +166,29 @@ def run_size(api, wfile, S, n_frames, host_steps, rounds):
         dt = time.perf_counter() - t
         return dt / k_steps, t_prop / (k_steps * S)
 
+    raw = RawArms(api, bank, S, steps, imu0, off0, P0) if raw_arms else None
+
     # warm-up of every shape
     bank_pass(4)
     net_pass(3)
     host_pass(1)
+    if raw:
+        raw.bank_pass(4)
+        raw.ceiling_pass(3)
     res = {"bank_step_s": [], "net_step_s": [], "host_step_s": [], "host_prop_per_seq_s": []}
     for _ in range(rounds):
         res["bank_step_s"].append(bank_pass(n_frames))
         res["net_step_s"].append(net_pass(n_frames))
+        if raw:
+            raw.timed_round(n_frames)
     hs, hp = host_pass(host_steps)
     res["host_step_s"].append(hs)
     res["host_prop_per_seq_s"].append(hp)
     for _ in range(rounds):
         res["bank_step_s"].append(bank_pass(n_frames))
         res["net_step_s"].append(net_pass(n_frames))
+        if raw:
+            raw.timed_round(n_frames)
 
     # filter-kernel time per step: CUDA kernel records of a profiled bank pass of its own
     from torch.profiler import ProfilerActivity, profile
@@ -181,11 +201,12 @@ def run_size(api, wfile, S, n_frames, host_steps, rounds):
             name = ev.name.split("filter_")[1].split("_kernel")[0]
             kern[name] = kern.get(name, 0.0) + ev.device_time / 1e6
     kern = {k: v / prof_frames for k, v in kern.items()}
+    bank_s, net_s, host_s = (float(np.median(res[k])) for k in ("bank_step_s", "net_step_s", "host_step_s"))
+    raw_row = raw.result(prof_frames, net_s) if raw else None
     bank.close()
     net.close()
-    bank_s, net_s, host_s = (float(np.median(res[k])) for k in ("bank_step_s", "net_step_s", "host_step_s"))
     filt = sum(kern.values())
-    return {
+    row = {
         "S": S, "frames": n_frames, "host_steps": host_steps,
         "bank_frames_per_s": S / bank_s, "host_loop_frames_per_s": S / host_s, "network_frames_per_s": S / net_s,
         "bank_over_host": host_s / bank_s,
@@ -196,6 +217,130 @@ def run_size(api, wfile, S, n_frames, host_steps, rounds):
         "host_propagate_ms_per_sequence": float(np.median(res["host_prop_per_seq_s"])) * 1e3,
         "bank_step_ms_all": [v * 1e3 for v in res["bank_step_s"]], "network_step_ms_all": [v * 1e3 for v in res["net_step_s"]],
     }
+    if raw_row:
+        row["raw"] = raw_row
+    return row
+
+
+def _union(intervals):
+    out = []
+    for a, b in sorted(intervals):
+        if out and a <= out[-1][1]:
+            out[-1][1] = max(out[-1][1], b)
+        else:
+            out.append([a, b])
+    return out
+
+
+def _overlap(intervals, union):
+    """Total length of `intervals` that lies inside the (sorted, disjoint) `union`."""
+    tot = 0.0
+    for a, b in intervals:
+        for c, d in union:
+            if c >= b:
+                break
+            tot += max(0.0, min(b, d) - max(a, c))
+    return tot
+
+
+class RawArms:
+    """The --raw arms on the bank of run_size: frame_raw from pinned raw frames, and the bare copy of the same bytes."""
+
+    def __init__(self, api, bank, S, steps, imu0, off0, P0):
+        import torch
+        from cuahn_vio_b200 import synthetic as Syn
+        self.api, self.lib, self.bank, self.S, self.steps = api, api.load_library(), bank, S, steps
+        self.state0, self.failed = (imu0, off0, P0), []     # slots whose filter diverged, per raw-bank pass
+        golden = np.load(os.path.join(ROOT, "tests", "golden", "preproc.npz"))
+        m1, m2 = api.undistort_init_maps(bool(golden[f"{RAW_CAMERA}_fisheye"]), golden[f"{RAW_CAMERA}_k"],
+                                         golden[f"{RAW_CAMERA}_d"])
+        bank.set_undistort_maps(RAW_ROWS, RAW_COLS, m1, m2)
+        uniq = np.stack([Syn.synthetic_raw_frame(900 + i, RAW_ROWS, RAW_COLS) for i in range(RAW_UNIQUE)])
+        # frame k of every slot: host[k % 2]; slot i shows unique frame (i + k) % RAW_UNIQUE
+        self.host = [torch.empty((S, RAW_ROWS, RAW_COLS), dtype=torch.uint8, pin_memory=True) for _ in range(2)]
+        for j, t in enumerate(self.host):
+            t.numpy()[:] = uniq[(np.arange(S) + j) % RAW_UNIQUE]
+        self.dev = torch.empty((S, RAW_ROWS, RAW_COLS), dtype=torch.uint8, device="cuda")
+        self.copy_stream = torch.cuda.Stream()
+        self.res = {"raw_step_s": [], "ceiling_step_s": []}
+
+    def bank_pass(self, frames_n):
+        import torch
+        bank, lib = self.bank, self.lib
+        bank.set_states(0, *self.state0)
+        torch.cuda.synchronize()
+        t = time.perf_counter()
+        for k in range(frames_n):
+            r, offsets, t0, t1 = self.steps[k]
+            if k:
+                assert lib.uahn_filter_propagate(bank._f, r.ctypes.data, offsets.ctypes.data, t0.ctypes.data, t1.ctypes.data) == 0
+            assert lib.uahn_filter_frame_raw(bank._f, None, self.host[k % 2].data_ptr(), RAW_COLS, 1, K_NET_COV, 2, None, None,
+                                             None, None, None, None) == 0
+        status = bank.wait()
+        dt = time.perf_counter() - t
+        self.failed.append(int((status != 0).sum()))
+        return dt / frames_n
+
+    def ceiling_pass(self, frames_n):
+        import torch
+        torch.cuda.synchronize()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        with torch.cuda.stream(self.copy_stream):
+            e0.record()
+            for k in range(frames_n):
+                self.dev.copy_(self.host[k % 2], non_blocking=True)      # cudaMemcpyAsync from pinned memory
+            e1.record()
+        e1.synchronize()
+        return e0.elapsed_time(e1) / 1e3 / frames_n
+
+    def timed_round(self, frames_n):
+        self.res["raw_step_s"].append(self.bank_pass(frames_n))
+        self.res["ceiling_step_s"].append(self.ceiling_pass(frames_n))
+
+    def result(self, prof_frames, net_s):
+        from torch.profiler import ProfilerActivity, profile
+        with profile(activities=[ProfilerActivity.CUDA]) as prof:
+            self.bank_pass(prof_frames)
+        remap = filt = h2d = 0.0
+        kernels, copies = [], []
+        for ev in prof.events():
+            if ev.device_type.name != "CUDA":
+                continue
+            span = (ev.time_range.start, ev.time_range.end)
+            if ev.name.startswith("Memcpy HtoD"):
+                h2d += ev.device_time / 1e6
+                copies.append(span)
+                continue
+            if ev.name.startswith("Memcpy") or ev.name.startswith("Memset"):
+                continue
+            kernels.append(span)
+            if "remap_bilinear_u8" in ev.name:
+                remap += ev.device_time / 1e6
+            elif "filter_" in ev.name:
+                filt += ev.device_time / 1e6
+        remap, filt, h2d = remap / prof_frames, filt / prof_frames, h2d / prof_frames
+        copy_total = sum(b - a for a, b in copies)
+        overlap = _overlap(copies, _union(kernels)) / copy_total if copy_total else 0.0
+        raw_s, ceil_s = (float(np.median(self.res[k])) for k in ("raw_step_s", "ceiling_step_s"))
+        raw_bytes = self.S * RAW_ROWS * RAW_COLS
+        remap_bytes = self.S * (RAW_ROWS * RAW_COLS + 224 * 320)      # raw frames read + undistorted frames written
+        bound = max(ceil_s, net_s + filt + remap)
+        return {
+            "raw_rows": RAW_ROWS, "raw_cols": RAW_COLS, "camera": RAW_CAMERA,
+            "raw_bank_frames_per_s": self.S / raw_s, "raw_bank_step_ms": raw_s * 1e3,
+            "raw_h2d_ceiling_ms_per_step": ceil_s * 1e3, "raw_h2d_ceiling_GB_per_s": raw_bytes / ceil_s / 1e9,
+            "h2d_device_ms_per_step_in_raw_bank": h2d * 1e3, "h2d_share_under_kernels": overlap,
+            "remap_kernel_ms_per_step": remap * 1e3, "remap_bytes_per_step": remap_bytes,
+            "remap_GB_per_s": remap_bytes / remap / 1e9 if remap else None,
+            "remap_hbm_bound_ms": remap_bytes / HBM_BYTES_PER_S * 1e3,
+            "remap_share_of_hbm_bound": (remap_bytes / HBM_BYTES_PER_S) / remap if remap else None,
+            "filter_kernel_ms_per_step": filt * 1e3, "network_step_ms": net_s * 1e3,
+            "compute_ms_per_step": (net_s + filt + remap) * 1e3, "raw_bound_ms": bound * 1e3,
+            "raw_step_over_bound": raw_s / bound,
+            "raw_bank_slots_failed_per_pass": self.failed,
+            "raw_bank_step_ms_all": [v * 1e3 for v in self.res["raw_step_s"]],
+            "raw_h2d_ceiling_ms_all": [v * 1e3 for v in self.res["ceiling_step_s"]],
+        }
 
 
 def main():
@@ -204,13 +349,14 @@ def main():
     ap.add_argument("--frames", type=int, default=64)
     ap.add_argument("--host-steps", type=int, default=4)
     ap.add_argument("--rounds", type=int, default=2)
+    ap.add_argument("--raw", action="store_true", help="add the raw-frame arms (uahn_filter_frame_raw, bare raw copy)")
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
     a = ap.parse_args()
     from cuahn_vio_b200 import api, build, weights
     build.build()
     wfile = weights.synthetic_weights_file(0)
     name, power = gpu_info()
-    rows = [run_size(api, wfile, S, a.frames, a.host_steps, a.rounds) for S in a.sizes]
+    rows = [run_size(api, wfile, S, a.frames, a.host_steps, a.rounds, a.raw) for S in a.sizes]
     line = json.dumps({"tool": "filter_bench", "gpu": name, "power_limit": power, "imu_hz": HZ_IMU, "camera_hz": HZ_CAM,
                        "precision": "bf16", "variant": "prior3", "max_iter": 1, "results": rows})
     print(line)
