@@ -68,11 +68,15 @@ class PropagatorConfig(C.Structure):
                 ("sigma_wb", C.c_double), ("sigma_ab", C.c_double), ("gravity_mag", C.c_double), ("imu_avg", C.c_int)]
 
     @classmethod
-    def make(cls, c_R_i, i_t_i2c, imu_avg: bool = True):
+    def make(cls, c_R_i, i_t_i2c, imu_avg: bool = True, sigma_w: float = 0.0, sigma_a: float = 0.0, sigma_wb: float = 0.0,
+             sigma_ab: float = 0.0, gravity_mag: float = 0.0):
+        """A sigma or gravity_mag <= 0 selects the reference default (Propagator.h:50-100)."""
         c = cls()
         c.c_R_i[:] = [float(v) for v in np.asarray(c_R_i, np.float64).reshape(9)]
         c.i_t_i2c[:] = [float(v) for v in np.asarray(i_t_i2c, np.float64).reshape(3)]
         c.imu_avg = int(imu_avg)
+        c.sigma_w, c.sigma_a, c.sigma_wb, c.sigma_ab = float(sigma_w), float(sigma_a), float(sigma_wb), float(sigma_ab)
+        c.gravity_mag = float(gravity_mag)
         return c
 
 

@@ -29,8 +29,10 @@ def skew_x(w):                                   # quat_ops.h:141-145
 
 
 def ham_quat_update(rot_vec):                    # quat_ops.h:526-538
+    """The reference divides by the angle unconditionally (NaN at zero); an exactly zero angle takes the limit
+    sin(a/2)/a -> 1/2 instead, the library's documented deviation (csrc/ekf_math.h quat_update)."""
     ang = np.linalg.norm(rot_vec)
-    dqv = np.sin(ang * 0.5) * rot_vec / ang
+    dqv = (np.sin(ang * 0.5) / ang if ang != 0 else 0.5) * rot_vec
     M = np.eye(4) * np.cos(ang * 0.5)
     M[1:4, 1:4] += skew_x(-dqv)
     M[0, 1:4] = -dqv

@@ -9,6 +9,10 @@ Only tests/ may import this.  Follows, expression by expression (products left t
   StateHelper::propagate_Cov                           cuahn/src/state/StateHelper.cpp:28-32
   quaternion helpers                                   ov_core/src/utils/quat_ops.h:141-145,479-484,526-550,573-588
 
+Zero rotations: rotvec_2_ham_quat and jr_theta take the limits sin(a/2)/a -> 1/2 and J_r -> I at an exactly zero angle
+(n == 0 only), as csrc/ekf_math.h does.  The reference divides by the angle unconditionally (NaN there); the limit is
+the library's documented deviation.
+
 Parity pinning: none available from the reference (no tests, Eigen absent) — "parity unpinned"; tests/test_imu.py
 checks this restatement against finite differences of its own mean propagation and the C++ against this restatement.
 """
@@ -33,14 +37,20 @@ def rotvec_2_ham_quat(rv):                          # quat_ops.h:582-588
     n = np.linalg.norm(rv)
     q = np.empty(4)
     q[0] = np.cos(n * 0.5)
-    q[1:4] = np.sin(n * 0.5) * rv / n
+    q[1:4] = (np.sin(n * 0.5) / n if n != 0 else 0.5) * rv
     return q
 
 
 def jr_theta(th):                                   # quat_ops.h:573-580
     n = np.linalg.norm(th)
+    if n == 0:
+        return np.eye(3)
     S = skew_x(th)
     return np.eye(3) - (1 - np.cos(n)) / (n * n) * S + (n - np.sin(n)) / (n * n * n) * S @ S
+
+
+SIGMA_DEFAULTS = {"sigma_w": 1.6968e-04, "sigma_a": 2.0000e-3, "sigma_wb": 1.9393e-05, "sigma_ab": 3.0000e-03}  # Propagator.h:50-71
+GRAVITY_DEFAULT = 9.81                                                                                          # Propagator.h:100
 
 
 def noise_Q(sw=1.6968e-04, sa=2.0000e-3, swb=1.9393e-05, sab=3.0000e-03):     # Propagator.h:50-97
@@ -176,15 +186,29 @@ def predict_and_compute(imu, offsets, cRi, it, minus, plus, imu_avg=True, gravit
     return new_imu, new_off, F, Fw
 
 
-def propagate(imu, offsets, P, cRi, it, readings, time0, time1, **kw):
-    """Propagator.cpp:28-79 + StateHelper.cpp:28-32."""
+def plane_distance(imu, it):
+    """dc of predict_and_compute (Propagator.cpp:216): the camera's distance to the ground plane, which the corner
+    dynamics divide by."""
+    return (ham_quat_2_rot(imu[3:7]) @ (imu[0:3] + it))[2]
+
+
+def propagate(imu, offsets, P, cRi, it, readings, time0, time1, imu_avg=True, sigma_w=0.0, sigma_a=0.0, sigma_wb=0.0,
+              sigma_ab=0.0, gravity_mag=0.0, dc_trace=None):
+    """Propagator.cpp:28-79 + StateHelper.cpp:28-32.  The sigmas and gravity_mag resolve like uahn_propagator_config's
+    (resolve_config): a value <= 0 selects the reference default.  dc_trace (a list) receives plane_distance() of the
+    state entering every interval."""
     prop = select_imu_readings(readings, time0, time1)
-    Q = noise_Q()
+    given = {"sigma_w": sigma_w, "sigma_a": sigma_a, "sigma_wb": sigma_wb, "sigma_ab": sigma_ab}
+    sig = {k: v if v > 0 else SIGMA_DEFAULTS[k] for k, v in given.items()}
+    Q = noise_Q(sig["sigma_w"], sig["sigma_a"], sig["sigma_wb"], sig["sigma_ab"])
+    g = gravity_mag if gravity_mag > 0 else GRAVITY_DEFAULT
     P = P.astype(np.float64).copy()
     n = 0
     if len(prop) > 1:
         for i in range(len(prop) - 1):
-            imu, offsets, F, Fw = predict_and_compute(imu, offsets, cRi, it, prop[i], prop[i + 1], **kw)
+            if dc_trace is not None:
+                dc_trace.append(plane_distance(imu, it))
+            imu, offsets, F, Fw = predict_and_compute(imu, offsets, cRi, it, prop[i], prop[i + 1], imu_avg, g)
             P = F @ P @ F.T + Fw @ Q @ Fw.T
             n += 1
     return imu, offsets, P, n

@@ -3,7 +3,7 @@ restatement's Jacobians vs finite differences of its own mean propagation.  CPU 
 import numpy as np
 import pytest
 
-from oracle import imu_oracle as I
+from oracle import filter_oracle as F, imu_oracle as I
 
 
 @pytest.fixture(scope="module")
@@ -104,22 +104,63 @@ def test_jacobians_match_finite_differences():
             assert np.abs(num - F[rows, 15 + 3 * k + j]).max() < 2e-7
 
 
+def _propagate_both(api, c, state, readings, t0, t1):
+    """uahn_imu_propagate and filter_oracle.propagate from the same state → (host status, intervals, state arrays),
+    (oracle status, intervals, state)."""
+    st = api.EkfState.from_arrays(*state)
+    try:
+        rc, n = 0, api.imu_propagate(api.PropagatorConfig.make(**c), st, readings, t0, t1)
+    except api.UahnError as e:
+        rc, n = int(str(e).rsplit(" ", 1)[1]), 0
+    status, est, en, _ = F.propagate(state, readings, t0, t1, c)
+    return (rc, n, st.arrays()), (status, en, est)
+
+
 def test_propagate_matches_restatement_and_keeps_cov_psd(api):
     rng = np.random.default_rng(13)
     imu, off, P = _state(rng)
     cRi, it = _extrinsics(rng)
     r = _readings(rng, n=40)
-    cfg = api.PropagatorConfig.make(cRi, it, True)
-    st = api.EkfState.from_arrays(imu, off, P)
-    n = api.imu_propagate(cfg, st, r, 10.012, 10.1333)
-    imu2, off2, P2 = st.arrays()
-    ei, eo, eP, en = I.propagate(imu, off, P, cRi, it, r, 10.012, 10.1333)
+    (_, n, (imu2, off2, P2)), (_, en, (ei, eo, eP)) = _propagate_both(
+        api, {"c_R_i": cRi, "i_t_i2c": it, "imu_avg": 1}, (imu, off, P), r, 10.012, 10.1333)
     assert n == en and n >= 20
     assert np.abs(imu2 - ei).max() < 1e-12 and np.abs(off2 - eo).max() < 1e-12
     assert np.abs(P2 - eP).max() < 1e-12 * max(1.0, np.abs(eP).max())
+    st = api.EkfState.from_arrays(imu2, off2, P2)
+    cfg = api.PropagatorConfig.make(cRi, it, True)
     assert np.linalg.eigvalsh(0.5 * (P2 + P2.T)).min() > 0 and np.trace(P2) > np.trace(P)
     # the prior the network gets after propagation: offsets x 159.5 (VioManager.cpp:230-234)
     prior_px, prop = api.ekf_prior_px(st)
     assert np.allclose(prior_px, off2[:, :2].reshape(8) * 159.5) and np.abs(prior_px).max() > 1e-3
     with pytest.raises(api.UahnError):
         api.imu_propagate(cfg, st, r, 10.1, 10.1)          # same instant: the reference exits (Propagator.cpp:32-35)
+
+
+SCHEDULES = F.edge_schedules(np.random.default_rng(5))
+
+
+@pytest.mark.parametrize("config", ["A", "B"])
+@pytest.mark.parametrize("schedule", range(len(SCHEDULES)), ids=[s["name"] for s in SCHEDULES])
+def test_propagate_edge_schedules_match_restatement(api, config, schedule):
+    """uahn_imu_propagate (ekf_math.h on the host) against the numpy restatement over the schedules the filter-bank
+    tests give their slots: long gaps, no interpolation, de-duplication, empty and single-reading lists, t1 <= t0, an
+    exactly zero rate (the zero-angle limits) and a fast spin.  Configuration B sets every field of
+    uahn_propagator_config away from its default."""
+    rng = np.random.default_rng(100 + schedule)
+    c, p_scale = F.configs(rng)[config]
+    s = SCHEDULES[schedule]
+    imu, off, P = F.initial_state(rng, p_scale)
+    if s["zero_bg"]:
+        imu[13:16] = 0.0
+    (rc, n, (hi, ho, hP)), (status, en, (ei, eo, eP)) = _propagate_both(api, c, (imu, off, P), s["readings"], s["t0"], s["t1"])
+    assert rc == status and n == en
+    if status or n == 0:                       # t1 <= t0, or fewer than two selected readings: the state stays
+        assert np.array_equal(hi, imu) and np.array_equal(ho, off) and np.array_equal(hP, P)
+        assert s["name"] in ("empty", "single", "t1_eq_t0", "t1_lt_t0", "t1_nan")
+        return
+    assert np.isfinite(hi).all() and np.isfinite(hP).all() and np.isfinite(eP).all()
+    e_imu = (np.abs(hi - ei) / np.maximum(1.0, np.abs(ei))).max()
+    e_off = (np.abs(ho - eo) / np.maximum(1.0, np.abs(eo))).max()
+    e_P = np.abs(hP - eP).max() / np.abs(eP).max()
+    print(f"{s['name']} {config}: {n} intervals, imu {e_imu:.1e}, offsets {e_off:.1e}, P {e_P:.1e} (relative)")
+    assert e_imu <= 1e-13 and e_off <= 1e-13 and e_P <= 1e-13        # worst seen: 9e-16
