@@ -22,7 +22,8 @@ EXPORTED_SYMBOLS = [
     "uahn_stage_warp", "uahn_debug_read", "uahn_profile_enable", "uahn_profile_read", "uahn_stage_conv", "uahn_submit_batch", "uahn_submit_sequence",
     "uahn_wait", "uahn_stage_transfer", "uahn_variant", "uahn_show_error",
 ]
-PREPROC_SYMBOLS = ["uahn_undistort_init_maps", "uahn_set_undistort_maps", "uahn_load_raw_image", "uahn_stage_undistort"]
+PREPROC_SYMBOLS = ["uahn_undistort_init_maps", "uahn_set_undistort_maps", "uahn_submit_sequence_raw", "uahn_load_raw_image",
+                   "uahn_stage_undistort"]
 EKF_SYMBOLS = ["uahn_ekf_prior_px", "uahn_ekf_update", "uahn_ekf_reset_offsets", "uahn_ekf_iekf_frame",
                "uahn_imu_select_readings", "uahn_imu_predict_and_compute", "uahn_imu_propagate"]
 FILTER_SYMBOLS = ["uahn_filter_create", "uahn_filter_destroy", "uahn_filter_set_states", "uahn_filter_get_states",
@@ -190,6 +191,8 @@ def load_library(path: str | None = None):
     lib.uahn_undistort_init_maps.restype = i
     lib.uahn_set_undistort_maps.argtypes = [vp, i, i, vp, vp]
     lib.uahn_set_undistort_maps.restype = i
+    lib.uahn_submit_sequence_raw.argtypes = [vp, i, vp, C.c_size_t, vp, C.POINTER(_Rng), vp, vp]
+    lib.uahn_submit_sequence_raw.restype = i
     lib.uahn_load_raw_image.argtypes = [vp, vp, i, i, C.c_size_t, dbl]
     lib.uahn_load_raw_image.restype = i
     lib.uahn_stage_undistort.argtypes = [vp, vp, i, i, C.c_size_t, vp]
@@ -260,6 +263,21 @@ def ekf_prior_px(state: "EkfState"):
     return a, b
 
 
+def _strided_frames(raw, n, raw_shape):
+    """→ (array, row stride): [n, rows, cols] u8 whose frames sit rows * stride bytes apart, copied only if they do not.
+    raw_shape: the (raw_rows, raw_cols) of the maps set last, or None."""
+    raw = np.asarray(raw)
+    assert raw.dtype == np.uint8 and raw.ndim == 3 and raw.shape[0] == n, (raw.dtype, raw.shape)
+    rows, cols = raw.shape[1:]
+    # the library reads rows x cols of the maps' raw size: a smaller array would be read past its end
+    assert raw_shape is None or (rows, cols) == raw_shape, ((rows, cols), raw_shape)
+    s0, s1, s2 = raw.strides
+    if not (s2 == 1 and s1 >= cols and (n == 1 or s0 == rows * s1)):
+        raw = np.ascontiguousarray(raw)
+        s1 = cols
+    return raw, s1
+
+
 def _ptr(a):
     if a is None:
         return None
@@ -291,6 +309,8 @@ class Uahn:
         self._lib = load_library()
         self._h = C.c_void_p()
         self.variant, self.show_error, self.precision, self.max_batch = variant, show_error, precision, max_batch
+        self._raw_shape = None       # (raw_rows, raw_cols) of the maps set last
+        self._keep = []              # inputs and outputs of submit_sequence_raw, alive until wait()
         cfg = _Config(os.fsencode(weights_path), VARIANTS[variant], -1 if show_error is None else int(show_error),
                       PRECISIONS[precision], device, max_batch, stream)
         rc = self._lib.uahn_create(C.byref(cfg), C.byref(self._h))
@@ -333,6 +353,7 @@ class Uahn:
     def set_undistort_maps(self, raw_rows: int, raw_cols: int, map1: np.ndarray, map2: np.ndarray):
         m1, m2 = np.ascontiguousarray(map1, np.float32), np.ascontiguousarray(map2, np.float32)
         self._check(self._lib.uahn_set_undistort_maps(self._h, raw_rows, raw_cols, _ptr(m1), _ptr(m2)))
+        self._raw_shape = (raw_rows, raw_cols)
 
     def load_raw_image(self, raw: np.ndarray, time_stamp: float = 0.0):
         raw = np.ascontiguousarray(raw, np.uint8)
@@ -392,6 +413,25 @@ class Uahn:
         self._check(self._lib.uahn_submit_sequence(self._h, n_frames, _ptr(frames), _ptr(prior), C.byref(rng), _ptr(mean),
                                                    _ptr(cov)))
 
+    def submit_sequence_raw(self, raw, prior, seed=0, first_pair=0):
+        """submit_sequence with raw camera frames [n_frames, raw_rows, raw_cols] u8 (any row stride), undistorted on the
+        device with the maps of set_undistort_maps() → (mean [n_frames - 1, 8], cov [n_frames - 1, 8, 8]), filled when
+        wait() returns.  Numpy buffers are pageable, so the copies do not overlap the forward; for that, pass pinned
+        buffers to submit_sequence_raw_ptrs."""
+        raw, stride = _strided_frames(raw, np.asarray(raw).shape[0], self._raw_shape)
+        n = raw.shape[0] - 1
+        prior = None if prior is None else np.ascontiguousarray(prior, np.float32).reshape(n, 8)
+        mean, cov = np.empty((n, 8), np.float32), np.empty((n, 8, 8), np.float32)
+        self.submit_sequence_raw_ptrs(raw.shape[0], raw, stride, prior, mean, cov, seed, first_pair)
+        self._keep += [raw, prior, mean, cov]
+        return mean, cov
+
+    def submit_sequence_raw_ptrs(self, n_frames, raw, stride, prior, mean, cov, seed=0, first_pair=0):
+        """Pipelined submission of one sequence of raw frames (raw pinned-host addresses, `stride` bytes per raw row)."""
+        rng = _Rng(seed, first_pair, None)
+        self._check(self._lib.uahn_submit_sequence_raw(self._h, n_frames, _ptr(raw), stride, _ptr(prior), C.byref(rng),
+                                                       _ptr(mean), _ptr(cov)))
+
     def iekf_frame(self, state: "EkfState", max_iter: int = 1, K_net_Cov: float = 10.0, min_images: int = 10,
                    use_measurement: bool = True, seed: int = 0, pair_index: int | None = None,
                    iterative: "Uahn | None" = None):
@@ -406,6 +446,7 @@ class Uahn:
 
     def wait(self):
         self._check(self._lib.uahn_wait(self._h))
+        self._keep = []
 
     def synchronize(self):
         self._check(self._lib.uahn_synchronize(self._h))
@@ -642,16 +683,7 @@ class FilterBank:
 
     def _raw_frames(self, raw):
         """→ (array, row stride): [n, rows, cols] u8 whose frames sit rows * stride bytes apart, copied only if they do not."""
-        raw = np.asarray(raw)
-        assert raw.dtype == np.uint8 and raw.ndim == 3 and raw.shape[0] == self.n, (raw.dtype, raw.shape)
-        rows, cols = raw.shape[1:]
-        # the library reads rows x cols of the maps' raw size: a smaller array would be read past its end
-        assert self._raw_shape is None or (rows, cols) == self._raw_shape, ((rows, cols), self._raw_shape)
-        s0, s1, s2 = raw.strides
-        if not (s2 == 1 and s1 >= cols and (self.n == 1 or s0 == rows * s1)):
-            raw = np.ascontiguousarray(raw)
-            s1 = cols
-        return raw, s1
+        return _strided_frames(raw, self.n, self._raw_shape)
 
     def wait(self):
         """→ per-slot codes since the previous wait (0, ERR_STATE, ERR_INVALID)."""

@@ -178,6 +178,9 @@ struct uahn_handle {
   cudaEvent_t ev_in[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
   uint8_t *s_prev[2] = {nullptr, nullptr}, *s_curr[2] = {nullptr, nullptr}, *s_frames[2] = {nullptr, nullptr};
   float *s_prior[2] = {nullptr, nullptr}, *s_mean[2] = {nullptr, nullptr}, *s_cov[2] = {nullptr, nullptr};
+  // raw sequences (uahn_submit_sequence_raw): (max_batch + 1) packed raw frames per staging set, allocated by the first
+  // raw submission and dropped by uahn_set_undistort_maps when a larger raw size no longer fits
+  uint8_t* s_raw[2] = {nullptr, nullptr};
   uint64_t submit_count = 0;
   bool pipeline_ready = false;
   uint64_t auto_pair = 0;   // MC-dropout pair index of calls made with rng == NULL: fresh masks on every forward
@@ -697,6 +700,7 @@ void uahn_destroy(uahn_handle* h) {
   for (auto& sp : h->prof_spans) { cudaEventDestroy(sp.a); cudaEventDestroy(sp.b); }
   for (cudaEvent_t e : h->prof_pool) cudaEventDestroy(e);
   if (h->copy_stream) { cudaStreamSynchronize(h->copy_stream); cudaStreamDestroy(h->copy_stream); }
+  for (uint8_t* p : h->s_raw) if (p) cudaFree(p);
   for (int i = 0; i < 2; ++i) { if (h->ev_in[i]) cudaEventDestroy(h->ev_in[i]); if (h->ev_done[i]) cudaEventDestroy(h->ev_done[i]); }
   for (cudaGraphExec_t g : h->graphs) if (g) cudaGraphExecDestroy(g);
   if (h->h_rng) cudaFreeHost(h->h_rng);
@@ -781,23 +785,36 @@ int ensure_pipeline(uahn_handle* h) {
 }
 
 // One pipelined submission.  frames == nullptr: n independent pairs from prev / curr.  frames != nullptr: n + 1
-// consecutive frames, pair i = (frames[i], frames[i+1]) — each frame crosses PCIe once.
-int submit(uahn_handle* h, int n, const uint8_t* prev, const uint8_t* curr, const uint8_t* frames, const float* prior,
-           const uahn_rng* rng, float* mean, float* cov) {
+// consecutive frames, pair i = (frames[i], frames[i+1]) — each frame crosses PCIe once.  raw != nullptr: the same n + 1
+// frames as raw camera frames (`stride` bytes per row), undistorted on the handle's stream into the frames staging.
+int submit(uahn_handle* h, int n, const uint8_t* prev, const uint8_t* curr, const uint8_t* frames, const uint8_t* raw,
+           size_t stride, const float* prior, const uahn_rng* rng, float* mean, float* cov) {
   if (n <= 0 || n > h->cap) return h->fail(UAHN_ERR_INVALID, "n=%d outside [1, max_batch=%d]", n, h->cap);
   if (rng && rng->keep_masks) return h->fail(UAHN_ERR_UNSUPPORTED, "explicit masks are not supported by the pipelined entry points");
   if (h->cfg.variant != UAHN_VARIANT_FULL && !prior) return h->fail(UAHN_ERR_INVALID, "this variant needs a prior");
+  if (raw && !h->raw_rows) return h->fail(UAHN_ERR_STATE, "uahn_set_undistort_maps has not been called");
+  if (raw && (stride < (size_t)h->raw_cols || stride > (size_t)INT32_MAX))   // cudaMemcpy2DAsync takes int-range pitches
+    return h->fail(UAHN_ERR_INVALID, "row stride %zu outside [raw_cols=%d, 2^31)", stride, h->raw_cols);
   CK(cudaSetDevice(h->cfg.device));
   int rc = ensure_pipeline(h);
   if (rc) return rc;
-  if (frames && !h->s_frames[0])
+  if ((frames || raw) && !h->s_frames[0])
     for (int i = 0; i < 2; ++i)
       if ((rc = dev_alloc(h, &h->s_frames[i], (size_t)(h->cap + 1) * IMG_PIXELS))) return rc;
+  if (raw)
+    for (uint8_t*& p : h->s_raw)
+      if (!p) CK(cudaMalloc(&p, (size_t)(h->cap + 1) * h->raw_rows * h->raw_cols));
   const int k = (int)(h->submit_count & 1);
   cudaStream_t cs = h->copy_stream, st = h->stream;
   CK(cudaStreamWaitEvent(cs, h->ev_done[k], 0));   // staging set k is free again (never-recorded events are complete)
   const uint8_t *dp, *dc;
-  if (frames) {
+  if (raw) {
+    // the remap that last read s_raw[k] ran on the handle's stream before ev_done[k] was recorded
+    CK(cudaMemcpy2DAsync(h->s_raw[k], (size_t)h->raw_cols, raw, stride, (size_t)h->raw_cols, (size_t)(n + 1) * h->raw_rows,
+                         cudaMemcpyHostToDevice, cs));
+    dp = h->s_frames[k];
+    dc = h->s_frames[k] + IMG_PIXELS;
+  } else if (frames) {
     CK(cudaMemcpyAsync(h->s_frames[k], frames, (size_t)(n + 1) * IMG_PIXELS, cudaMemcpyHostToDevice, cs));
     dp = h->s_frames[k];
     dc = h->s_frames[k] + IMG_PIXELS;
@@ -810,6 +827,12 @@ int submit(uahn_handle* h, int n, const uint8_t* prev, const uint8_t* curr, cons
   if (prior) CK(cudaMemcpyAsync(h->s_prior[k], prior, (size_t)n * 8 * 4, cudaMemcpyHostToDevice, cs));
   CK(cudaEventRecord(h->ev_in[k], cs));
   CK(cudaStreamWaitEvent(st, h->ev_in[k], 0));
+  if (raw) {   // charged to the warp stage, like the cell-array fill
+    h->prof_begin(0);
+    LAUNCH(launch_remap_u8(h->s_raw[k], h->raw_rows, h->raw_cols, (size_t)h->raw_cols, n + 1, h->d_map1, h->d_map2,
+                           h->s_frames[k], st));
+    h->prof_end();
+  }
   rc = forward_any(h, n, dp, dc, prior ? h->s_prior[k] : nullptr, rng, nullptr, h->s_mean[k], h->s_cov[k], nullptr);
   if (rc) return rc;
   CK(cudaMemcpyAsync(mean, h->s_mean[k], (size_t)n * 8 * 4, cudaMemcpyDeviceToHost, st));
@@ -824,7 +847,7 @@ int uahn_submit_batch(uahn_handle* h, int n, const uint8_t* prev, const uint8_t*
                       const uahn_rng* rng, float* mean, float* cov) {
   if (!h) return UAHN_ERR_INVALID;
   if (!prev || !curr || !mean || !cov) return h->fail(UAHN_ERR_INVALID, "null buffer");
-  return submit(h, n, prev, curr, nullptr, prior, rng, mean, cov);
+  return submit(h, n, prev, curr, nullptr, nullptr, 0, prior, rng, mean, cov);
 }
 
 int uahn_submit_sequence(uahn_handle* h, int n_frames, const uint8_t* frames, const float* prior, const uahn_rng* rng,
@@ -832,7 +855,15 @@ int uahn_submit_sequence(uahn_handle* h, int n_frames, const uint8_t* frames, co
   if (!h) return UAHN_ERR_INVALID;
   if (!frames || !mean || !cov) return h->fail(UAHN_ERR_INVALID, "null buffer");
   if (n_frames < 2) return h->fail(UAHN_ERR_STATE, "HNet cannot inference! Only has one image!");   // HomographyNet.cpp:155-158
-  return submit(h, n_frames - 1, nullptr, nullptr, frames, prior, rng, mean, cov);
+  return submit(h, n_frames - 1, nullptr, nullptr, frames, nullptr, 0, prior, rng, mean, cov);
+}
+
+int uahn_submit_sequence_raw(uahn_handle* h, int n_frames, const uint8_t* raw, size_t stride, const float* prior,
+                             const uahn_rng* rng, float* mean, float* cov) {
+  if (!h) return UAHN_ERR_INVALID;
+  if (!raw || !mean || !cov) return h->fail(UAHN_ERR_INVALID, "null buffer");
+  if (n_frames < 2) return h->fail(UAHN_ERR_STATE, "HNet cannot inference! Only has one image!");   // HomographyNet.cpp:155-158
+  return submit(h, n_frames - 1, nullptr, nullptr, nullptr, raw, stride, prior, rng, mean, cov);
 }
 
 int uahn_wait(uahn_handle* h) {
@@ -935,12 +966,14 @@ int uahn_set_undistort_maps(uahn_handle* h, int raw_rows, int raw_cols, const fl
     return h->fail(UAHN_ERR_INVALID, "bad undistort maps / raw size %dx%d", raw_rows, raw_cols);
   CK(cudaSetDevice(h->cfg.device));
   CK(cudaStreamSynchronize(h->stream));
+  if (h->copy_stream) CK(cudaStreamSynchronize(h->copy_stream));   // raw submissions upload into s_raw there
   int rc;
   if (!h->d_map1) {
     if ((rc = dev_alloc(h, &h->d_map1, (size_t)IMG_PIXELS, false))) return rc;
     if ((rc = dev_alloc(h, &h->d_map2, (size_t)IMG_PIXELS, false))) return rc;
   }
   if ((size_t)raw_rows * raw_cols > (size_t)h->raw_rows * h->raw_cols) {
+    for (uint8_t*& p : h->s_raw) { if (p) cudaFree(p); p = nullptr; }   // the next raw submission allocates the new size
     if (h->h_raw) { cudaFreeHost(h->h_raw); h->h_raw = nullptr; }
     if ((rc = dev_alloc(h, &h->d_raw, (size_t)raw_rows * raw_cols, false))) return rc;
     CK(cudaMallocHost((void**)&h->h_raw, (size_t)raw_rows * raw_cols));

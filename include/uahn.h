@@ -139,7 +139,8 @@ UAHN_API int uahn_variant(const uahn_handle* h);    /* the resolved UAHN_VARIANT
 UAHN_API int uahn_show_error(const uahn_handle* h); /* the resolved show_error flag */
 
 /* Per-stage device timing (bench.py's roofline): when enabled, every forward brackets each kernel group with
- * CUDA events on the handle's stream.  Categories: 0 = warp/concat/pool + error map (HBM-bound),
+ * CUDA events on the handle's stream.  Categories: 0 = warp/concat/pool + error map + the remap of raw
+ * sequence submissions (HBM-bound),
  * 1 = conv stacks (tensor-bound), 2 = MC-head 5120->256 GEMMs (tensor-bound), 3 = FC8+DLT / MC expand / final.
  * uahn_profile_read synchronises, adds the elapsed ms of all finished groups into ms[4] / launches[4]
  * (accumulating since the last uahn_profile_enable(h, 1)) and returns UAHN_OK. */

@@ -25,8 +25,18 @@ extern "C" {
  * every output pixel; the target camera is fixed: f = 159.5, c = (159.5, 111.5) (CamBase.h:166-169). */
 UAHN_API int uahn_undistort_init_maps(int fisheye, const double* k4, const double* d4, float* map1, float* map2);
 
-/* Upload the maps (HOST pointers) and declare the raw frame size; enables uahn_load_raw_image. */
+/* Upload the maps (HOST pointers) and declare the raw frame size; enables uahn_load_raw_image and
+ * uahn_submit_sequence_raw.  Waits for the handle's enqueued work first: a submission already made keeps the old maps. */
 UAHN_API int uahn_set_undistort_maps(uahn_handle* h, int raw_rows, int raw_cols, const float* map1, const float* map2);
+
+/* uahn_submit_sequence with raw frames: raw holds n_frames HOST frames [n_frames][raw_rows][stride] of ONE sequence
+ * (stride >= raw_cols bytes).  Pair i = (remap(raw_i), remap(raw_{i+1})), cv::remap-exact with the handle's maps.
+ * Everything after the remap (priors, rng numbering, outputs, the uahn_wait contract, at most two in flight) is
+ * exactly uahn_submit_sequence's.  UAHN_ERR_STATE without maps.  The upload of submission i+1 runs on the copy
+ * stream under the remap and forward of submission i; raw should be pinned for the copy to overlap.  Device memory:
+ * two staging buffers of (max_batch + 1) raw frames, allocated by the first call. */
+UAHN_API int uahn_submit_sequence_raw(uahn_handle* h, int n_frames, const uint8_t* raw, size_t stride,
+                                      const float* prior, const uahn_rng* rng, float* mean, float* cov);
 
 /* undistort_and_resize_img + load_current_img (VioManager.cpp:181-188) in one call: raw is CV_8UC1 raw_rows x raw_cols
  * with `stride` bytes per row, borrowed for the duration of the call.  prev <- curr, curr <- remap(raw). */
